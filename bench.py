@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: env-steps/sec of the batched Pioneer 6-DoF reach env on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--envs-per-gpu E] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -71,6 +71,9 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-steps-per-proc", type=int, default=0,
                     help="reference arm: env-steps per process per bench step (0 = sized for ~20 s in total)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0: obs, reward, flags) "
+                         "as DIR/<name>.npy, so that two builds can be compared output for output on the same inputs")
     return ap.parse_args()
 
 
@@ -440,6 +443,28 @@ def make_buffers(torch, env, n, device, seed, ring=FRAGMENT):
     return actions, obs_ring, reward, flags
 
 
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Write each array of `arrays` (name -> [N, ...], one row per env) as out_dir/<name>.npy: float64 stays float64, every
+    other dtype becomes float32.  When the rows do not fit in DUMP_BYTES_MAX, the same fixed, seeded sample of rows is
+    taken from every array and the sampled env indices are written as env_index.npy (float64)."""
+    import numpy as np
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v[:1].nbytes for v in arrays.values())
+    if n * row_bytes > DUMP_BYTES_MAX:
+        keep = (DUMP_BYTES_MAX - 4096 * (len(arrays) + 1)) // (row_bytes + 8)       # 4 KiB for each .npy header
+        rows = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(v))
+
+
 def pre_age(torch, env, limit, seed):
     """Give every env a random age in [0, limit): the timed region then runs the steady-state mix of a long rollout, with
     n / limit TimeLimit truncations + in-kernel Philox auto-resets per step, instead of `limit` reset-free steps."""
@@ -523,6 +548,10 @@ def ours_arm(args):
     total_envs = n * world
     value = total_envs * args.steps / (kernel_ms_max / 1e3)
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs and rank == 0:                      # the last timed step's slot, before later timings reuse it
+        last = per_frag[-1][1] - 1
+        dump_outputs(args.dump_outputs, {"obs": obs_ring[last].cpu(), "reward": reward[last].cpu(),
+                                         "flags": flags[last].cpu()})
     # the path's one exchange: episode statistics, once per iteration (distributed.IterationSync).  Within a node it is ONE
     # kernel per rank over NVLink peer memory (pnr_iteration_sync: snapshot + stores into every rank's window + flags + merge),
     # replayed from a CUDA graph; the NCCL form (snapshot kernel + all_gather_into_tensor + merge kernel, eager) is timed

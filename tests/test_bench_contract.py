@@ -37,6 +37,53 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_dump_outputs_types_and_cap(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(0)
+    arrays = {"obs": rng.normal(size=(100, 137)).astype(np.float32), "reward": rng.normal(size=100),
+              "flags": rng.integers(0, 4, size=100, dtype=np.uint8)}
+    bench.dump_outputs(str(tmp_path / "all"), arrays)
+    got = {k: np.load(tmp_path / "all" / f"{k}.npy") for k in ("obs", "reward", "flags")}
+    assert not (tmp_path / "all" / "env_index.npy").exists()
+    assert got["obs"].dtype == np.float32 and got["reward"].dtype == np.float64 and got["flags"].dtype == np.float32
+    for k in arrays:
+        assert np.array_equal(got[k], arrays[k])
+    # over the cap: the same seeded rows of every array, and their indices
+    monkeypatch.setattr(bench, "DUMP_BYTES_MAX", 30 * 1024 + 4096 * 4)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["env_index.npy", "flags.npy", "obs.npy", "reward.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES_MAX
+    rows = np.load(tmp_path / "a" / "env_index.npy")
+    assert rows.dtype == np.float64 and 0 < len(rows) < 100 and np.all(np.diff(rows) > 0)
+    for k in arrays:
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert np.array_equal(a, b) and np.array_equal(a, arrays[k][rows.astype(int)].astype(a.dtype))
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs: the same arguments give the same inputs, so two runs write identical outputs."""
+    import numpy as np
+    n = 4096
+    for d in ("a", "b"):
+        out = subprocess.run([sys.executable, "bench.py", "--steps", "21", "--warmup", "3", "--no-sweep", "--no-cpu-baseline",
+                              "--no-extras", "--envs-per-gpu", str(n), "--dump-outputs", str(tmp_path / d)],
+                             cwd=ROOT, capture_output=True, text=True, timeout=900)
+        assert out.returncode == 0, out.stderr[-3000:]
+        assert _one_json_line(out.stdout)["steps"] == 21
+    shapes = {"obs": (n, 137), "reward": (n,), "flags": (n,)}
+    assert sorted(p.name for p in (tmp_path / "a").iterdir()) == sorted(f"{k}.npy" for k in shapes)
+    for k, shape in shapes.items():
+        a, b = np.load(tmp_path / "a" / f"{k}.npy"), np.load(tmp_path / "b" / f"{k}.npy")
+        assert a.shape == shape and a.dtype == np.float32 and np.isfinite(a).all()
+        assert np.array_equal(a, b), k
+    flags = np.load(tmp_path / "a" / "flags.npy")
+    assert set(np.unique(flags)) <= {0.0, 1.0, 2.0, 3.0}
+
+
 @pytest.mark.gpu
 def test_gpu_arm_line():
     out = subprocess.run([sys.executable, "bench.py", "--steps", "30", "--warmup", "3", "--no-sweep", "--no-cpu-baseline",
