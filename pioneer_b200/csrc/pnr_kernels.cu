@@ -81,8 +81,9 @@ extern "C" int pnr_debug_trace(unsigned long long* out_host) {
 // pnr_filter_apply feeds, so the 548 B/env observation is never re-read.  Every warp normalises the columns it owns
 // while the tile is still in shared memory: a joint warp runs one column pass (lane = one of its 30 changing
 // columns, 32 rows, float64 sum / sum of squares of x - mean), the task warp normalises its 11 tail values in
-// registers and keeps per-lane float partial sums; the 36 constant columns are normalised once per CTA and their
-// statistics are added analytically by block 0.  The raw r / cos r / sin r the task warp needs for the forward
+// registers and keeps per-lane float partial sums over one step's tiles, added to float64 per-lane sums in shared memory
+// at the start of the next step; the 36 constant columns are normalised once per CTA and their statistics are added
+// analytically by block 0.  The raw r / cos r / sin r the task warp needs for the forward
 // kinematics travel through a small scratch area next to the tile buffers (the tile copy gets normalised).
 template <int ARITH, int OBS_MODE, bool OBSTACLES, bool FILTER>
 __global__ void __launch_bounds__(PNR_STEP_THREADS, FILTER ? PNR_STEP_MIN_CTAS_FILTER : PNR_STEP_MIN_CTAS)
@@ -135,6 +136,7 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
     float f_mean = 0.f, f_inv = 0.f;
     double f_sum = 0.0, f_sq = 0.0;
     float t_sum[11], t_sq[11];
+    __shared__ double f_tacc[FILTER ? 22 * 32 : 1];               // task warp: float64 sum / sum of squares per lane, per tail column
     if (FILTER) {
         if (part < 3) {
             // lanes 0..5 -> column blocks 0..2 (r, cos r, sin r), lanes 6..29 -> blocks 9..20; blocks 3..8 are constant
@@ -154,6 +156,8 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
         } else {
 #pragma unroll
             for (int i = 0; i < 11; ++i) { t_sum[i] = 0.f; t_sq[i] = 0.f; }
+#pragma unroll
+            for (int i = 0; i < 22; ++i) f_tacc[i * 32 + lane] = 0.0;   // each lane owns its column of f_tacc
         }
     }
 
@@ -194,6 +198,18 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
         __syncthreads();
         t_idx = blockIdx.x;
         issue_loads(t_idx, act_s);
+        if (FILTER && part == 3) {
+            // the task warp's float partials cover the tiles of ONE step; each lane adds them to its own float64 sums in
+            // shared memory (no double registers to spare at 128), so a fragment sums the same per-step values that single
+            // steps do and the float rounding does not grow with the fragment length.  Done here, while the joint warps
+            // integrate the first tile of this step, the task warp would otherwise only wait for them.
+#pragma unroll
+            for (int i = 0; i < 11; ++i) {
+                f_tacc[i * 32 + lane] += (double)t_sum[i];
+                f_tacc[(11 + i) * 32 + lane] += (double)t_sq[i];
+                t_sum[i] = 0.f; t_sq[i] = 0.f;
+            }
+        }
     }
     for (; t_idx < n_tiles; t_idx += stride) {
         const int64_t env_raw = t_idx * PNR_TILE_ENVS + lane;
@@ -419,15 +435,15 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
         } else {
 #pragma unroll
             for (int i = 0; i < 11; ++i) {
-                float a = t_sum[i], b = t_sq[i];
+                double a = f_tacc[i * 32 + lane] + (double)t_sum[i], b = f_tacc[(11 + i) * 32 + lane] + (double)t_sq[i];
 #pragma unroll
                 for (int ofs = 16; ofs > 0; ofs >>= 1) {
                     a += __shfl_xor_sync(PNR_FULL_MASK, a, ofs);
                     b += __shfl_xor_sync(PNR_FULL_MASK, b, ofs);
                 }
                 if (lane == 0) {
-                    atomicAdd(&f_slot[1 + 126 + i], (double)a);
-                    atomicAdd(&f_slot[1 + PNR_OBS_DIM + 126 + i], (double)b);
+                    atomicAdd(&f_slot[1 + 126 + i], a);
+                    atomicAdd(&f_slot[1 + PNR_OBS_DIM + 126 + i], b);
                 }
             }
             if (blockIdx.x == 0 && lane == 0) atomicAdd(&f_delta[0], (double)N * multi.n_steps);
