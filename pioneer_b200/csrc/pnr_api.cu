@@ -556,7 +556,7 @@ extern "C" int pnr_step(pnr_handle* h, const float* actions, float* obs, float* 
 extern "C" int pnr_step_many(pnr_handle* h, int32_t n_steps, const float* actions, int64_t action_stride, float* obs,
                              int64_t obs_stride, float* reward, uint8_t* done, void* stream) {
     if (!h || n_steps < 0) return pnr_fail(PNR_ERR_INVALID, "pnr_step_many: bad argument");
-    // The whole fragment is ONE launch (PnrMulti): every CTA (kinematic kernel; a CTA barrier between the steps) or warp
+    // The whole fragment is ONE launch (PnrMulti): every CTA (kinematic kernel; each tile's steps back to back) or warp
     // (dynamic kernel; the env state stays in registers) runs the n_steps steps on its own tiles -- tiles never depend on each
     // other, so there is no launch gap and no grid-wide wait between the steps.  PNR_NO_FUSE=1 (developer knob): one launch
     // per step, overlapped by programmatic dependent launch only.

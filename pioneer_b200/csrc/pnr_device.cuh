@@ -185,9 +185,9 @@ __device__ __forceinline__ void pnr_bulk_wait_read() {      // returns once at m
 __device__ __forceinline__ void pnr_pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pnr_pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-// A rollout fragment in ONE launch of the kinematic step kernel (pnr_step_many): the CTA keeps its tiles and runs n_steps
-// consecutive steps on them -- tiles never depend on each other, so no grid-wide synchronisation is needed between the
-// steps, only a CTA barrier.  Step s reads actions + s * act_stride and writes obs + s * obs_stride (floats), reward / done
+// A rollout fragment in ONE launch of the kinematic step kernel (pnr_step_many): the CTA runs the n_steps consecutive steps
+// of each of its tiles before it takes the next tile -- tiles never depend on each other, so no grid-wide synchronisation is
+// needed between the steps.  Step s reads actions + s * act_stride and writes obs + s * obs_stride (floats), reward / done
 // + s * N.  n_steps = 1 for an ordinary pnr_step.
 struct PnrMulti { int32_t n_steps; int64_t act_stride, obs_stride; };
 

@@ -14,47 +14,62 @@
 //                                from the tile), reward / done / TimeLimit (:151-165), episode statistics,
 //                                auto-reset (reset_world, :76-105), observation tail, planes X0, X1,
 //                                reward / done outputs, and the TMA bulk store of the finished tile
-// The two roles run as a producer / consumer pipeline over TWO tile buffers, coupled only by named barriers:
+// A rollout fragment (PnrMulti, n_steps steps in one launch) runs TILE-OUTER, STEP-INNER: a CTA takes a tile, runs all
+// n_steps steps on it, then takes its next tile.  Every warp reads its state planes once when a tile starts, keeps the env
+// state in registers across the steps -- in the layout of its planes: r, v | a of its two joints for a joint warp, target,
+// t | potential, return for the task warp -- and writes it back once after the tile's last step.
+// The CTA's work items, (tile, step) in that order, alternate between TWO tile buffers and run as a producer / consumer
+// pipeline coupled only by named barriers:
 //   HEAD[b]  joint warps arrive once r, cos r, sin r of their joints are in buffer b; the task warp waits on it
-//   DONE[b]  joint warps arrive once all their columns and planes are written; the task warp waits, then stores
-//   FREE[b]  the task warp arrives once the bulk store of buffer b has been read; joint warps wait before reuse
+//   DONE[b]  joint warps arrive once all their columns (and, after a tile's last step, planes) are written; the task warp
+//            waits, then stores
+//   FREE[b]  the task warp arrives once the bulk store of the item before this one has been read AND this item's resets
+//            are published (below); joint warps wait before they write the head of the next item into buffer b
 //   JOINT    (OBSTACLES only) the three joint warps among themselves, once their heads are in the tile: each then sums the
 //            penetration depths of its share of the capsule table into shared memory; the task warp adds the three partials
 //            behind DONE and only then writes reward, return and episode statistics
-// so the joint warps of a CTA work on tile i+1 while its task warp finishes tile i (before: 49 % of stall samples
-// were joint warps parked at a CTA-wide barrier).  Each warp prefetches its own planes of the CTA's next tile.
+// Step s + 1 of an env depends on step s only through an auto-reset, and only the task warp decides it.  Before it arrives
+// at FREE it publishes the item's reset mask and, for the reset lanes, the new joint angles (and box) in shared memory.  The
+// joint warps integrate the next step of the tile from their registers before they wait on FREE and redo it from the
+// reset state for the (rare) masked lanes after it.  So no barrier spans the whole CTA: the joint warps work on item i+1
+// while the task warp finishes item i, across step and tile boundaries alike.  A ragged last tile (a byte count that is
+// no multiple of 16, so no bulk store) is streamed out by the task warp alone, under the same protocol.
 // Grid = min(tiles, resident CTAs of the whole GPU); grid-stride over tiles.
 // ---------------------------------------------------------------------------------------------
-// In-kernel auto-reset of ONE env by the task warp after the tile is complete: new joint angles and target from
-// the Philox stream, a = v = 0, potential = 0, elapsed = 0 written over all eight planes of the env; in
-// PNR_OBS_AUTORESET mode the env's observation row is replaced by the first observation of the new episode.
-// Rare (once per episode), so deliberately not inlined: keeps registers and code out of the hot loop.
-// In-kernel auto-reset of ONE env by the task warp after the tile is complete: new joint angles and target from
-// the Philox stream, a = v = 0, potential = 0, elapsed = 0 written over all eight planes of the env; in
-// PNR_OBS_AUTORESET mode the env's observation row is replaced by the first observation of the new episode.
+// In-kernel auto-reset of ONE env by the task warp once its step is decided: new joint angles, target and box from the Philox
+// stream (a = v = 0, potential = 0, elapsed = 0).  The joint angles, and the box of the random-box variant, go to the lane's
+// column of `pub` (stride 32) for the joint warps' next step of the tile, the box also to its plane; after the tile's LAST
+// step the env's eight state planes are written too.  In PNR_OBS_AUTORESET mode the env's observation row is replaced by the
+// first observation of the new episode.  Returns the new target.
 // Rare (once per episode), so deliberately not inlined: keeps registers and code out of the hot loop.
 // (Tried and dropped: drawing the next episode as soon as the TimeLimit hit is known, before the task warp waits for the
 // joint warps -- the divergent Philox lane delays the whole task warp, which IS the critical path there: 11.8 -> 12.9 us
 // per 65,536-env step.)
-template <int OBS_MODE>
-__device__ __noinline__ void pnr_auto_reset(const PnrParams& p, float4* __restrict__ state, int64_t env, uint64_t tickdom,
-                                            float* __restrict__ row) {
-    const int64_t N = p.n_envs;
+template <int OBS_MODE, bool OBSTACLES>
+__device__ __noinline__ float4 pnr_auto_reset(const PnrParams& p, float4* __restrict__ state, int64_t env, uint64_t tickdom,
+                                              float* __restrict__ row, float* __restrict__ pub, bool last) {
     PnrEnv s;
     float q[PNR_DOF], tg[3], box[5];
     pnr_reset_draws(p, p.env_id_base + env, pnr_reset_key(p, tickdom), q, tg, box);
     pnr_reset_env(s, q, tg);
-    pnr_store_env(state, N, env, s);
     pnr_store_box(p, env, box);
+#pragma unroll
+    for (int i = 0; i < PNR_DOF; ++i) pub[i * 32] = q[i];
+    if (OBSTACLES && p.random_box >= 0) {
+#pragma unroll
+        for (int i = 0; i < 5; ++i) pub[(PNR_DOF + i) * 32] = box[i];
+    }
+    if (last) pnr_store_env(state, p.n_envs, env, s);
     if (OBS_MODE == PNR_OBS_AUTORESET) {
         PnrPose o;
         pnr_pose<true>(p, s, o);                              // fresh joint angles lie inside the limits
         pnr_pack_obs_dyn<true>(p, row, s, o, s.pot);
     }
+    return make_float4(tg[0], tg[1], tg[2], 0.f);
 }
 
 #ifdef PNR_TRACE
-// developer instrumentation (python -m pioneer_b200.build --trace): per-CTA phase timestamps of the first tile
+// developer instrumentation (python -m pioneer_b200.build --trace): per-CTA phase timestamps of the first work items
 #define PNR_TRACE_SLOTS 12
 #define PNR_TRACE_CTAS 2048
 #define PNR_TRACE_ITERS 4
@@ -81,10 +96,9 @@ extern "C" int pnr_debug_trace(unsigned long long* out_host) {
 // pnr_filter_apply feeds, so the 548 B/env observation is never re-read.  Every warp normalises the columns it owns
 // while the tile is still in shared memory: a joint warp runs one column pass (lane = one of its 30 changing
 // columns, 32 rows, float64 sum / sum of squares of x - mean), the task warp normalises its 11 tail values in
-// registers and keeps per-lane float partial sums over one step's tiles, added to float64 per-lane sums in shared memory
-// at the start of the next step; the 36 constant columns are normalised once per CTA and their statistics are added
-// analytically by block 0.  The raw r / cos r / sin r the task warp needs for the forward
-// kinematics travel through a small scratch area next to the tile buffers (the tile copy gets normalised).
+// registers and adds them, per lane and per step, to float64 sums in shared memory; the 36 constant columns are normalised
+// once per CTA and their statistics are added analytically by block 0.  The raw r / cos r / sin r the task warp needs for
+// the forward kinematics travel through a small scratch area next to the tile buffers (the tile copy gets normalised).
 template <int ARITH, int OBS_MODE, bool OBSTACLES, bool FILTER>
 __global__ void __launch_bounds__(PNR_STEP_THREADS, FILTER ? PNR_STEP_MIN_CTAS_FILTER : PNR_STEP_MIN_CTAS)
 pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state, const float* __restrict__ actions,
@@ -92,6 +106,11 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
                 PnrStats* __restrict__ stats, uint32_t tick, uint32_t domain, const float* __restrict__ f_applied,
                 double* __restrict__ f_delta, float f_clip, const PnrMulti multi) {
     extern __shared__ __align__(128) float tiles[];           // PNR_STEP_BUFS tiles: the bulk store of one drains
+    // the task warp's resets of its current item, for the joint warps' next step of the tile: lane mask, joint angles of
+    // env `lane` at s_pub[j * 32 + lane]; OBSTACLES: rows 6..10 hold the tile's current per-env box (centre x y, half
+    // extents x y z), written by joint warp 0 when a tile starts and by the task warp at a reset
+    __shared__ uint32_t s_reset;
+    __shared__ float s_pub[(OBSTACLES ? PNR_DOF + 5 : PNR_DOF) * 32];
     const int lane = threadIdx.x & 31;                        // while the next is being filled
     const int part = threadIdx.x >> 5;                        // warp-uniform role
     float* tile = tiles;
@@ -135,7 +154,6 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
     int f_col = 0;
     float f_mean = 0.f, f_inv = 0.f;
     double f_sum = 0.0, f_sq = 0.0;
-    float t_sum[11], t_sq[11];
     __shared__ double f_tacc[FILTER ? 22 * 32 : 1];               // task warp: float64 sum / sum of squares per lane, per tail column
     if (FILTER) {
         if (part < 3) {
@@ -155,82 +173,84 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             }
         } else {
 #pragma unroll
-            for (int i = 0; i < 11; ++i) { t_sum[i] = 0.f; t_sq[i] = 0.f; }
-#pragma unroll
             for (int i = 0; i < 22; ++i) f_tacc[i * 32 + lane] = 0.0;   // each lane owns its column of f_tacc
         }
     }
 
-    // software pipeline: every warp loads its own planes of the NEXT tile while it works on the current one
-    float4 ld4; float2 ld2, ld_act = make_float2(0.f, 0.f);
-    // (state planes through L2 only: with programmatic dependent launch this CTA may have started on an SM before the previous
-    // step finished elsewhere; nothing is re-read, so L1 would buy nothing)
-    auto issue_loads = [&](int64_t tile_idx, const float* __restrict__ act) {
+    // the env state of the current tile in registers, in plane layout (joint warp: r r v v | a a; task warp: target t | potential
+    // return); software pipeline: the next tile's planes and the next item's action are loaded while this item is worked on.
+    // (State planes through L2 only: with programmatic dependent launch this CTA may have started on an SM before the previous
+    // step finished elsewhere; nothing is re-read, so L1 would buy nothing.)
+    float4 st4, ld4;
+    float2 st2, ld2, ld_act = make_float2(0.f, 0.f);
+    auto load_planes = [&](int64_t tile_idx) {
         const int64_t e_raw = tile_idx * PNR_TILE_ENVS + lane;
         const int64_t e = e_raw < N ? e_raw : N - 1;
         if (part < 3) {
             ld4 = __ldcg(rv_plane + e);
             ld2 = __ldcg(a_plane + e);
-            ld_act = pnr_ld_stream(reinterpret_cast<const float2*>(act + e * PNR_DOF) + part);
         } else {
             ld4 = __ldcg(x0_plane + e);
             ld2 = __ldcg(x1_plane + e);
         }
     };
+    auto load_act = [&](int64_t tile_idx, int32_t s) {
+        if (part < 3) {
+            const int64_t e_raw = tile_idx * PNR_TILE_ENVS + lane;
+            const int64_t e = e_raw < N ? e_raw : N - 1;
+            ld_act = pnr_ld_stream(reinterpret_cast<const float2*>(actions + (int64_t)s * multi.act_stride + e * PNR_DOF) + part);
+        }
+    };
     pnr_pdl_wait();                                           // the previous step's state planes are complete and visible
-    issue_loads(t_idx, actions);
+    load_planes(t_idx);
+    load_act(t_idx, 0);
     PNR_MARK(2);
     int buf = 0;
-    int64_t iter = 0;                                         // tiles this CTA has started
+    int64_t iter = 0;                                         // work items this CTA has started
+    int32_t step = 0;                                         // step of the fragment (PnrMulti; 1 step for pnr_step)
 
-    // n_steps consecutive steps on this CTA's own tiles (PnrMulti; 1 for an ordinary step).  Between two steps the warps of
-    // the CTA meet at a barrier: the task warp may have reset an env of the tile, which rewrites planes the joint warps
-    // are about to load again.
-    for (int32_t step = 0; step < multi.n_steps; ++step) {
-    const bool more_steps = step + 1 < multi.n_steps;
-    // this step's buffers (launch-uniform: the bases stay in the constant bank)
-    const float* __restrict__ const act_s = actions + (int64_t)step * multi.act_stride;
-    float* __restrict__ const obs_s = obs + (int64_t)step * multi.obs_stride;
-    float* __restrict__ const reward_s = reward + (int64_t)step * N;
-    uint8_t* __restrict__ const done_s = done + (int64_t)step * N;
-    const uint32_t tick_s = tick + (uint32_t)step;
-    if (step > 0) {
-        __syncthreads();
-        t_idx = blockIdx.x;
-        issue_loads(t_idx, act_s);
-        if (FILTER && part == 3) {
-            // the task warp's float partials cover the tiles of ONE step; each lane adds them to its own float64 sums in
-            // shared memory (no double registers to spare at 128), so a fragment sums the same per-step values that single
-            // steps do and the float rounding does not grow with the fragment length.  Done here, while the joint warps
-            // integrate the first tile of this step, the task warp would otherwise only wait for them.
-#pragma unroll
-            for (int i = 0; i < 11; ++i) {
-                f_tacc[i * 32 + lane] += (double)t_sum[i];
-                f_tacc[(11 + i) * 32 + lane] += (double)t_sq[i];
-                t_sum[i] = 0.f; t_sq[i] = 0.f;
-            }
-        }
-    }
-    for (; t_idx < n_tiles; t_idx += stride) {
+    for (;;) {
+        const bool last = step + 1 == multi.n_steps;          // the tile's last step: its state goes back to the planes
+        const int64_t next_tile = last ? t_idx + stride : t_idx;
+        const bool more = next_tile < n_tiles;                // CTA-uniform: another item follows on this CTA
+        // this step's buffers (launch-uniform bases)
+        float* __restrict__ const obs_s = obs + (int64_t)step * multi.obs_stride;
+        float* __restrict__ const reward_s = reward + (int64_t)step * N;
+        uint8_t* __restrict__ const done_s = done + (int64_t)step * N;
+        const uint32_t tick_s = tick + (uint32_t)step;
         const int64_t env_raw = t_idx * PNR_TILE_ENVS + lane;
         const bool active = env_raw < N;
-        const int64_t env = active ? env_raw : N - 1;       // tail lanes shadow the last env, stores masked
+        const int64_t env = active ? env_raw : N - 1;         // tail lanes shadow the last env, stores masked
         const int64_t rows_left = N - t_idx * PNR_TILE_ENVS;
         const int rows_valid = rows_left < PNR_TILE_ENVS ? (int)rows_left : PNR_TILE_ENVS;
-        const float4 c4 = ld4;
-        const float2 c2 = ld2, c_act = ld_act;
-        if (t_idx + stride < n_tiles) issue_loads(t_idx + stride, act_s);
+        if (step == 0) { st4 = ld4; st2 = ld2; }              // a new tile: its state, read once
+        const float2 c_act = ld_act;
+        float4 box_a = make_float4(0.f, 0.f, 0.f, 0.f);       // OBSTACLES, joint warp 0: the new tile's boxes
+        float box_z = 0.f;
+        if (OBSTACLES && part == 0 && step == 0 && p.random_box >= 0) { box_a = p.box_a[env]; box_z = p.box_z[env]; }
+        if (more) {
+            if (last) load_planes(next_tile);
+            load_act(next_tile, last ? 0 : step + 1);
+        }
 
         float r1[2], v1[2], sn[2], cs[2];
         if (part < 3) {
             // --- act(): integrate with the PREVIOUS action (one-step actuation delay); registers only
-            pnr_integrate_joint<ARITH>(p, vmax0, rlo0, rhi0, c2.x, c4.z, c4.x, v1[0], r1[0]);
-            pnr_integrate_joint<ARITH>(p, vmax1, rlo1, rhi1, c2.y, c4.w, c4.y, v1[1], r1[1]);
-            pnr_sincos_fast(r1[0], sn[0], cs[0]);             // r is inside the joint limits: fast path
-            pnr_sincos_fast(r1[1], sn[1], cs[1]);
+            auto advance = [&]() {
+                pnr_integrate_joint<ARITH>(p, vmax0, rlo0, rhi0, st2.x, st4.z, st4.x, v1[0], r1[0]);
+                pnr_integrate_joint<ARITH>(p, vmax1, rlo1, rhi1, st2.y, st4.w, st4.y, v1[1], r1[1]);
+                pnr_sincos_fast(r1[0], sn[0], cs[0]);         // r is inside the joint limits: fast path
+                pnr_sincos_fast(r1[1], sn[1], cs[1]);
+            };
+            advance();
             PNR_MARK(3);
-            if (iter >= PNR_STEP_BUFS) pnr_bar_sync2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf);   // buffer reusable
+            if (iter >= 1) pnr_bar_sync2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf);   // buffer reusable, resets published
             PNR_MARK(4);
+            if (step > 0 && ((s_reset >> lane) & 1u)) {       // the task warp reset this env after the previous step
+                st4 = make_float4(s_pub[j0 * 32 + lane], s_pub[(j0 + 1) * 32 + lane], 0.f, 0.f);
+                st2 = make_float2(0.f, 0.f);
+                advance();
+            }
             pnr_pack_joint_head(rowj, r1[0], sn[0], cs[0]);
             pnr_pack_joint_head(rowj + 1, r1[1], sn[1], cs[1]);
             if (FILTER) {                                      // the raw values for the task warp's forward kinematics
@@ -247,7 +267,7 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
 
         bool do_reset = false;
         // OBSTACLES: what the task warp carries across the DONE barrier (the penalty is summed from the joint warps' partials)
-        float d_rew = 0.f, d_ep = 0.f, d_pot = 0.f;
+        float d_rew = 0.f;
         int32_t d_t = 0;
         bool d_done = false, d_reached = false;
         if (part < 3) {
@@ -255,20 +275,28 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             const bool fast = !p.trig_slow && fmaxf(fabsf(c_act.x), fabsf(c_act.y)) <= PNR_TRIG_FAST_LIMIT;
             pnr_pack_joint_rest(rowj, rlo0, rhi0, r1[0], v1[0], c_act.x, fast);
             pnr_pack_joint_rest(rowj + 1, rlo1, rhi1, r1[1], v1[1], c_act.y, fast);
-            if (active) {
-                rv_plane[env] = make_float4(r1[0], r1[1], v1[0], v1[1]);
-                a_plane[env] = c_act;
+            st4 = make_float4(r1[0], r1[1], v1[0], v1[1]);
+            st2 = c_act;
+            if (last && active) {
+                rv_plane[env] = st4;
+                a_plane[env] = st2;
             }
             if (OBSTACLES) {
                 // capsule penetration depths, the capsule table split over the three joint warps (on the task warp alone
                 // they were the CTA's critical path: 59 % of the stall samples were joint warps parked at DONE).  Every
                 // joint's sin/cos is needed: the joint warps meet once their heads are in the tile.
+                if (part == 0 && step == 0) {
+                    s_pub[6 * 32 + lane] = box_a.x; s_pub[7 * 32 + lane] = box_a.y;
+                    s_pub[8 * 32 + lane] = box_a.z; s_pub[9 * 32 + lane] = box_a.w; s_pub[10 * 32 + lane] = box_z;
+                }
                 pnr_bar_sync<PNR_BAR_JOINT, 3 * 32>();
                 const float* head = FILTER ? srow : row;
                 PnrSinCos sc;
 #pragma unroll
                 for (int i = 0; i < PNR_DOF; ++i) { sc.cs[i] = head[6 + i]; sc.sn[i] = head[12 + i]; }
-                pen[(buf * 3 + part) * 32 + lane] = pnr_contact_depth(p, sc, pnr_load_box(p, env), part, 3);
+                const float bz = s_pub[10 * 32 + lane];
+                const PnrBox rb = {s_pub[6 * 32 + lane], s_pub[7 * 32 + lane], bz, s_pub[8 * 32 + lane], s_pub[9 * 32 + lane], bz};
+                pen[(buf * 3 + part) * 32 + lane] = pnr_contact_depth(p, sc, rb, part, 3);
             }
             if (FILTER) {                                      // column pass over this warp's 30 changing columns
                 __syncwarp();
@@ -300,10 +328,10 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             const float* head = FILTER ? srow : row;           // raw r | cos r | sin r of this env
 #pragma unroll
             for (int i = 0; i < PNR_DOF; ++i) { o.cs[i] = head[6 + i]; o.sn[i] = head[12 + i]; }
-            const float tgt[3] = {c4.x, c4.y, c4.z};
-            int32_t t = __float_as_int(c4.w);
-            const float pot_old = c2.x;
-            float ep_ret = c2.y;
+            const float tgt[3] = {st4.x, st4.y, st4.z};
+            int32_t t = __float_as_int(st4.w);
+            const float pot_old = st2.x;
+            float ep_ret = st2.y;
             pnr_fk_tip(p, o.sn, o.cs, o.ptr);
             const float dx = tgt[0] - o.ptr[0], dy = tgt[1] - o.ptr[1], dz = tgt[2] - o.ptr[2];
             o.dist = sqrtf(fmaf(dx, dx, fmaf(dy, dy, dz * dz)));
@@ -328,7 +356,7 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             const uint8_t flags = (is_done ? PNR_DONE : 0) | ((timeout && !reached) ? PNR_TRUNCATED : 0);
             if (active) done_s[env] = flags;
             if (OBSTACLES) {                                   // the penalty arrives with DONE: reward, return and statistics wait
-                d_rew = rew; d_ep = ep_ret; d_pot = pot_new; d_t = t; d_done = is_done; d_reached = reached;
+                d_rew = rew; d_t = t; d_done = is_done; d_reached = reached;
             } else {
                 ep_ret = __fadd_rn(ep_ret, rew);
                 if (active) reward_s[env] = rew;
@@ -338,85 +366,96 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             // observation tail: pointer, target, difference, distance, potential (terminal values)
             float tail[11] = {o.ptr[0], o.ptr[1], o.ptr[2], tgt[0], tgt[1], tgt[2],
                               tgt[0] - o.ptr[0], tgt[1] - o.ptr[1], tgt[2] - o.ptr[2], o.dist, pot_new};
-            if (FILTER) {                                      // normalise in registers, per-lane partial statistics
+            if (FILTER) {                                      // normalise in registers, float64 statistics per lane
 #pragma unroll
                 for (int i = 0; i < 11; ++i) {
                     const float d = tail[i] - f_applied[126 + i];
-                    if (active) { t_sum[i] += d; t_sq[i] = fmaf(d, d, t_sq[i]); }
+                    if (active) {
+                        const double e = (double)d;
+                        f_tacc[i * 32 + lane] += e;
+                        f_tacc[(11 + i) * 32 + lane] = fma(e, e, f_tacc[(11 + i) * 32 + lane]);
+                    }
                     tail[i] = fminf(fmaxf(d * f_applied[PNR_OBS_DIM + 126 + i], -f_clip), f_clip);
                 }
             }
 #pragma unroll
             for (int i = 0; i < 11; ++i) row[126 + i] = tail[i];
 
-            if (active) {
-                x0_plane[env] = make_float4(tgt[0], tgt[1], tgt[2], __int_as_float(t));
-                if (!OBSTACLES) x1_plane[env] = make_float2(pot_new, ep_ret);
+            st4.w = __int_as_float(t);
+            st2 = make_float2(pot_new, ep_ret);                // OBSTACLES: the return is completed behind DONE
+            if (last && active) {
+                x0_plane[env] = st4;
+                if (!OBSTACLES) x1_plane[env] = st2;
             }
-            do_reset = is_done && active && (p.auto_reset != 0);   // handled after B2 (rare)
+            do_reset = is_done && active && (p.auto_reset != 0);   // handled after DONE (rare)
         }
         PNR_MARK(6);
         pnr_fence_async_smem();                               // generic-proxy tile writes -> async proxy
-        const bool bulk = pnr_tile_is_bulk(rows_valid);       // CTA-uniform
-        if (!bulk) __syncthreads();                           // ragged last tile of the grid: everybody streams it out
-        else if (part < 3) pnr_bar_arrive2<PNR_BAR_DONE, PNR_STEP_THREADS>(buf);
-        else pnr_bar_sync2<PNR_BAR_DONE, PNR_STEP_THREADS>(buf);   // tile complete, joint planes stored
+        if (part < 3) pnr_bar_arrive2<PNR_BAR_DONE, PNR_STEP_THREADS>(buf);
+        else pnr_bar_sync2<PNR_BAR_DONE, PNR_STEP_THREADS>(buf);   // tile complete (joint planes stored after a last step)
         PNR_MARK(7);
 
-        if (OBSTACLES && part == 3) {                         // obstacle variant: capsule penetration penalty, then the deferred writes
-            const float* pb = pen + buf * PNR_PEN_FLOATS + lane;
-            const float depth = (pb[0] + pb[32]) + pb[64];
-            const float rew = __fsub_rn(d_rew, __fmul_rn(p.contact_penalty, depth));
-            const float ep_ret = __fadd_rn(d_ep, rew);
-            if (active) {
-                reward_s[env] = rew;
-                x1_plane[env] = make_float2(d_pot, ep_ret);
-            }
-            pnr_episode_stats(stats, d_done && active, d_reached && active, ep_ret, d_t, lane);
-        }
         if (part == 3) {
-            // rare: auto-reset (reset_world, :76-105).  Only the auto-reset observation mode rewrites the row, so only there
-            // does the reset have to precede the tile's store; terminal mode resets AFTER handing the tile to the copy engine
-            const bool any_reset = __any_sync(PNR_FULL_MASK, do_reset);
-            if (OBS_MODE == PNR_OBS_AUTORESET && any_reset) {
-                if (do_reset) pnr_auto_reset<OBS_MODE>(p, state, env, pnr_tickdom(tick_s, domain), row);
-                pnr_fence_async_smem();
-                __syncwarp();
+            if (OBSTACLES) {                                  // capsule penetration penalty, then the deferred writes
+                const float* pb = pen + buf * PNR_PEN_FLOATS + lane;
+                const float depth = (pb[0] + pb[32]) + pb[64];
+                const float rew = __fsub_rn(d_rew, __fmul_rn(p.contact_penalty, depth));
+                st2.y = __fadd_rn(st2.y, rew);
+                if (active) {
+                    reward_s[env] = rew;
+                    if (last) x1_plane[env] = st2;
+                }
+                pnr_episode_stats(stats, d_done && active, d_reached && active, st2.y, d_t, lane);
             }
-            if (bulk) {
+            // rare: auto-reset (reset_world, :76-105).  Only the auto-reset observation mode rewrites the row, so only there
+            // does the reset have to precede the tile's store; terminal mode resets AFTER handing the tile to the copy engine.
+            // Either way before FREE: that is where the joint warps pick the new episode up.
+            const unsigned reset_mask = __ballot_sync(PNR_FULL_MASK, do_reset);
+            float* const pub = s_pub + lane;
+            const uint64_t tickdom = pnr_tickdom(tick_s, domain);
+            if (OBS_MODE == PNR_OBS_AUTORESET && reset_mask) {
+                if (do_reset) {
+                    const float4 tg = pnr_auto_reset<OBS_MODE, OBSTACLES>(p, state, env, tickdom, row, pub, last);
+                    st4 = make_float4(tg.x, tg.y, tg.z, __int_as_float(0));
+                    st2 = make_float2(0.f, 0.f);
+                }
+                pnr_fence_async_smem();
+            }
+            __syncwarp();
+            if (pnr_tile_is_bulk(rows_valid)) {
                 if (lane == 0) {
                     pnr_bulk_store(obs_s + t_idx * (int64_t)PNR_TILE_FLOATS, tile,
                                    (uint32_t)(rows_valid * PNR_OBS_DIM * sizeof(float)));
                     pnr_bulk_commit();
-                    // every store but the one just committed has finished READING its buffer: the previous tile's
-                    // buffer is free again (only signalled if a tile that will reuse it exists)
-                    if (iter >= 1) pnr_bulk_wait_read<1>();
+                    // every store but the one just committed has finished READING its buffer: the previous item's
+                    // buffer is free again
+                    pnr_bulk_wait_read<1>();
                 }
-                __syncwarp();
-                if (iter >= 1 && (t_idx + stride < n_tiles || more_steps)) pnr_bar_arrive2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf ^ 1);
+            } else {                                          // ragged last tile of the grid: the task warp streams it out
+                pnr_emit_tile_manual(tile, obs_s + t_idx * (int64_t)PNR_TILE_FLOATS, rows_valid, lane, 32);
+                if (lane == 0) pnr_bulk_wait_read<0>();
             }
-            if (OBS_MODE != PNR_OBS_AUTORESET && any_reset && do_reset)
-                pnr_auto_reset<OBS_MODE>(p, state, env, pnr_tickdom(tick_s, domain), row);
+            if (OBS_MODE != PNR_OBS_AUTORESET && do_reset) {
+                const float4 tg = pnr_auto_reset<OBS_MODE, OBSTACLES>(p, state, env, tickdom, row, pub, last);
+                st4 = make_float4(tg.x, tg.y, tg.z, __int_as_float(0));
+                st2 = make_float2(0.f, 0.f);
+            }
+            if (lane == 0) s_reset = reset_mask;
+            __syncwarp();
+            if (more) pnr_bar_arrive2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf ^ 1);
         }
         PNR_MARK(8);
         PNR_TRACE_NEXT();
-        if (!bulk) {                                          // ragged last tile: all 128 threads stream it out
-            if (part == 3 && iter >= 1 && more_steps) {       // (another step follows: keep the buffer protocol going)
-                if (lane == 0) pnr_bulk_wait_read<0>();
-                __syncwarp();
-                pnr_bar_arrive2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf ^ 1);
-            }
-            __syncthreads();
-            pnr_emit_tile_manual(tile, obs_s + t_idx * (int64_t)PNR_TILE_FLOATS, rows_valid, threadIdx.x, PNR_STEP_THREADS);
-        }
-        buf ^= 1;                                             // next tile goes into the other buffer
+        if (!more) break;
+        t_idx = next_tile;
+        step = last ? 0 : step + 1;
+        buf ^= 1;                                             // next item goes into the other buffer
         ++iter;
         tile = tiles + buf * PNR_TILE_FLOATS;
         row = tile + lane * PNR_OBS_DIM;
         rowj = row + j0;
         if (FILTER) srow = scratch + buf * PNR_FSCRATCH_FLOATS + lane * PNR_FSCRATCH_STRIDE;
     }
-    }                                                         // steps
     if (FILTER && f_delta != nullptr) {                       // column statistics of this CTA's rows, into copy blockIdx % SLOTS
         double* f_slot = f_delta + (size_t)(blockIdx.x & (PNR_FILTER_SLOTS - 1)) * PNR_FILTER_DELTA_LEN;
         if (part < 3) {
@@ -435,7 +474,7 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
         } else {
 #pragma unroll
             for (int i = 0; i < 11; ++i) {
-                double a = f_tacc[i * 32 + lane] + (double)t_sum[i], b = f_tacc[(11 + i) * 32 + lane] + (double)t_sq[i];
+                double a = f_tacc[i * 32 + lane], b = f_tacc[(11 + i) * 32 + lane];
 #pragma unroll
                 for (int ofs = 16; ofs > 0; ofs >>= 1) {
                     a += __shfl_xor_sync(PNR_FULL_MASK, a, ofs);
@@ -704,13 +743,14 @@ cudaError_t pnr_launch_step(const PnrParams& p, int device, int arith, int obs_m
         cudaError_t e = pnr_prepare(k, smem, &resident);
         if (e != cudaSuccess) return e;
     }
-    // Resident CTAs per SM, measured on B200 (profiles/r01_v4_cta_sweep.md): long grid-stride runs stream best with
-    // 4 CTAs per SM (87 % of the HBM copy peak at 2M envs against 80 % with 6), short ones need all 6 to fill the GPU.
+    // Resident CTAs per SM, measured on B200 (profiles/r03_step_65536.md): with the steps of a fragment pipelined per tile,
+    // 4 CTAs per SM stream best from 2,048 tiles on (131,072 envs: 14.2 us per step against 15.1 with 5 or 6; 65,536 envs:
+    // 7.9 against 8.2 with 6); smaller grids keep 6 per SM so that up to 888 tiles run at once.
     static int sms_of[PNR_MAX_DEVICES] = {};
     int& dev_sms = sms_of[device % PNR_MAX_DEVICES];
     if (dev_sms == 0) cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, device);
     const int64_t n_tiles = (p.n_envs + PNR_TILE_ENVS - 1) / PNR_TILE_ENVS;
-    int per_sm = n_tiles >= 16384 ? 4 : (n_tiles >= 8192 ? 5 : 6);
+    int per_sm = n_tiles >= 2048 ? 4 : 6;
     if (const char* e = getenv("PNR_CTAS_PER_SM")) per_sm = atoi(e) > 0 ? atoi(e) : per_sm;   // developer knob
     int cap = per_sm * dev_sms < resident ? per_sm * dev_sms : resident;
     const int64_t grid = pnr_grid_for(p.n_envs, PNR_TILE_ENVS, cap);
@@ -719,7 +759,8 @@ cudaError_t pnr_launch_step(const PnrParams& p, int device, int arith, int obs_m
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     // programmatic dependent launch pays where the launch tail is a visible share of the step (65,536 envs: 13.2 -> 11.8 us);
-    // on long grids the early-resident successor only takes SM slots from this grid (1,048,576 envs: 146 -> 151 us)
+    // on long grids the early-resident successor only takes SM slots from this grid (1,048,576 envs: 146 -> 151 us).
+    // One launch per fragment: fragments are timed the same with and without it (profiles/r03_step_65536.md)
     attr[0].val.programmaticStreamSerializationAllowed = (pnr_pdl_enabled() && n_tiles <= 8192) ? 1 : 0;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, k, p, state, actions, obs, reward, done, stats, tick, domain, f_applied, f_delta, f_clip, multi);
