@@ -137,7 +137,7 @@ def load(build_if_missing: bool = True) -> C.CDLL:
     if _lib is not None:
         return _lib
     path = _build.LIB_PATH
-    override = os.environ.get("PIONEER_B200_LIB")        # developer builds (e.g. the -DPNR_TRACE library)
+    override = os.environ.get("PIONEER_B200_LIB")        # another build of the library (A/B comparisons)
     if override:
         path, build_if_missing = override, False
     if build_if_missing:

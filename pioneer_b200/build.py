@@ -53,18 +53,12 @@ def _stale() -> bool:
     return _built_hash(LIB_PATH) != _source_hash()
 
 
-TRACE_LIB_PATH = os.path.join(LIB_DIR, "libpioneer_b200_trace.so")
-
-
-def build(force: bool = False, verbose: bool = False, trace: bool = False) -> str:
-    """trace=True: developer build with per-CTA phase timestamps (-DPNR_TRACE) next to the product library;
-    select it with PIONEER_B200_LIB=<path>.
-
-    Safe when several processes (the ranks of a torchrun job) import the package at once: one of them builds under a
+def build(force: bool = False, verbose: bool = False) -> str:
+    """Safe when several processes (the ranks of a torchrun job) import the package at once: one of them builds under a
     file lock into a temporary file that is renamed into place, the others wait and find the library fresh."""
     import fcntl
-    out = TRACE_LIB_PATH if trace else LIB_PATH
-    if not trace and not force and not _stale():
+    out = LIB_PATH
+    if not force and not _stale():
         return LIB_PATH
     os.makedirs(LIB_DIR, exist_ok=True)
     extra = os.environ.get("PNR_EXTRA_NVCC_FLAGS", "").split()     # developer experiments (e.g. -DPNR_STEP_MIN_CTAS=6)
@@ -78,7 +72,7 @@ def build(force: bool = False, verbose: bool = False, trace: bool = False) -> st
                 return LIB_PATH
             nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
             tmp = f"{out}.tmp.{os.getpid()}"
-            cmd = [nvcc] + NVCC_FLAGS + extra + (["-DPNR_TRACE"] if trace else []) + (["-Xptxas", "-v"] if verbose else []) \
+            cmd = [nvcc] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) \
                 + [f'-DPNR_SRC_HASH="{_source_hash()}"'] + _sources() + ["-o", tmp]
             proc = subprocess.run(cmd, capture_output=True, text=True)
             if proc.returncode != 0:
@@ -94,4 +88,4 @@ def build(force: bool = False, verbose: bool = False, trace: bool = False) -> st
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv, trace="--trace" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))

@@ -556,31 +556,24 @@ extern "C" int pnr_step(pnr_handle* h, const float* actions, float* obs, float* 
 extern "C" int pnr_step_many(pnr_handle* h, int32_t n_steps, const float* actions, int64_t action_stride, float* obs,
                              int64_t obs_stride, float* reward, uint8_t* done, void* stream) {
     if (!h || n_steps < 0) return pnr_fail(PNR_ERR_INVALID, "pnr_step_many: bad argument");
+    if (n_steps == 0) return PNR_OK;
     // The whole fragment is ONE launch (PnrMulti): every CTA (kinematic kernel; each tile's steps back to back) or warp
     // (dynamic kernel; the env state stays in registers) runs the n_steps steps on its own tiles -- tiles never depend on each
-    // other, so there is no launch gap and no grid-wide wait between the steps.  PNR_NO_FUSE=1 (developer knob): one launch
-    // per step, overlapped by programmatic dependent launch only.
-    static const bool fuse_on = getenv("PNR_NO_FUSE") == nullptr;
-    if (fuse_on && n_steps > 1) {
+    // other, so there is no launch gap and no grid-wide wait between the steps.  A single step reads no stride.
+    if (n_steps > 1) {
         if ((reinterpret_cast<uintptr_t>(obs) & 15) || ((obs_stride * sizeof(float)) & 15))
             return pnr_fail(PNR_ERR_INVALID, "pnr_step_many: obs and obs_stride * 4 must be multiples of 16 bytes");
         if ((action_stride * sizeof(float)) & 7)
             return pnr_fail(PNR_ERR_INVALID, "pnr_step_many: action_stride * 4 must be a multiple of 8 bytes");
-        return pnr_step_impl(h, actions, obs, reward, done, stream, PnrMulti{n_steps, action_stride, obs_stride});
     }
-    for (int32_t t = 0; t < n_steps; ++t) {
-        int rc = pnr_step_impl(h, actions + (int64_t)t * action_stride, obs + (int64_t)t * obs_stride,
-                               reward + (int64_t)t * h->n_envs, done + (int64_t)t * h->n_envs, stream);
-        if (rc != PNR_OK) return rc;
-    }
-    return PNR_OK;
+    return pnr_step_impl(h, actions, obs, reward, done, stream, PnrMulti{n_steps, action_stride, obs_stride});
 }
 
 extern "C" int pnr_observe_done(pnr_handle* h, const uint8_t* done, float* obs, float* terminal_obs, void* stream) {
     if (!h || !done || !obs) return pnr_fail(PNR_ERR_INVALID, "pnr_observe_done: null argument");
     PnrDeviceGuard guard(h->device);
     const bool fused = h->filt_fused != 0;
-    PNR_CUDA(pnr_launch_observe_done(h->params, h->state, done, obs, terminal_obs, fused ? h->filt_applied : nullptr,
+    PNR_CUDA(pnr_launch_observe_done(h->params, h->device, h->state, done, obs, terminal_obs, fused ? h->filt_applied : nullptr,
                                      (fused && h->filt_fused_update) ? h->filt_delta : nullptr, (float)h->filt_clip,
                                      (cudaStream_t)stream));
     h->launches += 1;
@@ -594,8 +587,7 @@ static int pnr_host_setup(pnr_handle* h) {
         cudaError_t e;
         if (!h->host_stream && (e = cudaStreamCreateWithFlags(&h->host_stream, cudaStreamNonBlocking)) != cudaSuccess) return e;
         if (!h->copy_stream1 && (e = cudaStreamCreateWithFlags(&h->copy_stream1, cudaStreamNonBlocking)) != cudaSuccess) return e;
-        if (!getenv("PNR_HOST_ONE_STREAM") && !h->copy_stream2 &&  // developer knob: one copy engine for the observations
-            (e = cudaStreamCreateWithFlags(&h->copy_stream2, cudaStreamNonBlocking)) != cudaSuccess) return e;
+        if (!h->copy_stream2 && (e = cudaStreamCreateWithFlags(&h->copy_stream2, cudaStreamNonBlocking)) != cudaSuccess) return e;
         if (!h->host_order_event && (e = cudaEventCreateWithFlags(&h->host_order_event, cudaEventDisableTiming)) != cudaSuccess) return e;
         for (auto& sl : h->slot) {
             for (cudaEvent_t* ev : {&sl.kernel_done, &sl.copy1_done, &sl.copy2_done})
@@ -641,7 +633,7 @@ extern "C" int pnr_step_host_begin(pnr_handle* h, const float* actions, float* o
     if (rc != PNR_OK) return rc;
     const float* src = sl.obs;
     if (layout == PNR_HOST_COMPACT) {
-        PNR_CUDA(pnr_launch_compact_obs(sl.obs, sl.compact, h->n_envs, s));
+        PNR_CUDA(pnr_launch_compact_obs(h->device, sl.obs, sl.compact, h->n_envs, s));
         h->launches += 1;
         src = sl.compact;
     }
@@ -649,18 +641,15 @@ extern "C" int pnr_step_host_begin(pnr_handle* h, const float* actions, float* o
     // The observation copy is what bounds this call (PCIe).  Two copy engines working on the two halves keep the link
     // fuller than one; reward / done ride on the first stream.
     const size_t total = n * (size_t)width;
-    const size_t half = h->copy_stream2 ? (n / 2) * (size_t)width : total;
+    const size_t half = (n / 2) * (size_t)width;
     PNR_CUDA(cudaStreamWaitEvent(h->copy_stream1, sl.kernel_done, 0));
-    if (half < total) {
-        PNR_CUDA(cudaStreamWaitEvent(h->copy_stream2, sl.kernel_done, 0));
-        PNR_CUDA(cudaMemcpyAsync(obs + half, src + half, (total - half) * sizeof(float), cudaMemcpyDeviceToHost, h->copy_stream2));
-        PNR_CUDA(cudaEventRecord(sl.copy2_done, h->copy_stream2));
-    }
+    PNR_CUDA(cudaStreamWaitEvent(h->copy_stream2, sl.kernel_done, 0));
+    PNR_CUDA(cudaMemcpyAsync(obs + half, src + half, (total - half) * sizeof(float), cudaMemcpyDeviceToHost, h->copy_stream2));
+    PNR_CUDA(cudaEventRecord(sl.copy2_done, h->copy_stream2));
     if (half > 0) PNR_CUDA(cudaMemcpyAsync(obs, src, half * sizeof(float), cudaMemcpyDeviceToHost, h->copy_stream1));
     PNR_CUDA(cudaMemcpyAsync(reward, sl.reward, n * sizeof(float), cudaMemcpyDeviceToHost, h->copy_stream1));
     PNR_CUDA(cudaMemcpyAsync(done, sl.done, n, cudaMemcpyDeviceToHost, h->copy_stream1));
     PNR_CUDA(cudaEventRecord(sl.copy1_done, h->copy_stream1));
-    if (half >= total) PNR_CUDA(cudaEventRecord(sl.copy2_done, h->copy_stream1));
     sl.busy = true;
     h->host_next ^= 1;
     h->host_inflight += 1;

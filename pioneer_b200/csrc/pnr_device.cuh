@@ -233,6 +233,31 @@ struct PnrStats {
     uint32_t tick_offset;
     uint32_t seed_lo, seed_hi;      // the reset generator's key (pnr_create / pnr_seed)
 };
+// The statistics window as the host reads it, PNR_STATS_LEN doubles: episodes, sum of returns, sum of lengths, sum of squared
+// returns, max return, min return, env-steps, reached.
+__device__ __forceinline__ double pnr_stats_read(const PnrStats* stats, int i) {
+    switch (i) {
+        case 0: return stats->episodes;
+        case 1: return stats->sum_return;
+        case 2: return stats->sum_length;
+        case 3: return stats->sum_return_sq;
+        case 4: return (double)pnr_ordered_to_float(stats->max_return_ord);
+        case 5: return (double)pnr_ordered_to_float(stats->min_return_ord);
+        case 6: return stats->env_steps;
+        default: return stats->reached;
+    }
+}
+__device__ __forceinline__ void pnr_stats_clear(PnrStats* stats) {
+    stats->episodes = stats->sum_return = stats->sum_length = stats->sum_return_sq = stats->reached = 0.0;
+    stats->env_steps = 0.0;
+    stats->max_return_ord = pnr_float_to_ordered(-INFINITY);
+    stats->min_return_ord = pnr_float_to_ordered(INFINITY);
+}
+// how ranks combine field i of their windows, in rank order: MAX of the max returns, MIN of the min returns, SUM of the rest
+// (and of whatever follows the window in a packed vector, the observation filter's sums)
+__device__ __forceinline__ double pnr_stats_combine(int i, double acc, double x) {
+    return i == 4 ? fmax(acc, x) : (i == 5 ? fmin(acc, x) : acc + x);
+}
 // tickdom = domain << 32 | host call counter: ONE 64-bit argument for the rare, non-inlined reset paths
 __device__ __forceinline__ PnrResetKey pnr_reset_key(const PnrParams& p, uint64_t tickdom) {
     PnrResetKey k;

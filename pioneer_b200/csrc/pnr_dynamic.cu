@@ -6,14 +6,6 @@
 #include <cstdlib>
 #include "pnr_dynamic_kernel.cuh"
 
-static int pnr_dyn_resident(const void* fn) {
-    int dev = 0, sms = 0, per_sm = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PNR_DYN_THREADS, PNR_DYN_SMEM);
-    return sms * (per_sm < 1 ? 1 : per_sm);
-}
-
 cudaError_t pnr_launch_step_dynamic(const PnrParams& p, int device, int obs_mode, float4* state, const float* actions,
                                     float* obs, float* reward, uint8_t* done, PnrStats* stats, uint32_t tick, uint32_t domain,
                                     const float* f_applied, double* f_delta, float f_clip, PnrMulti multi, cudaStream_t stream) {
@@ -32,20 +24,13 @@ cudaError_t pnr_launch_step_dynamic(const PnrParams& p, int device, int obs_mode
     Kern kern = stepping ? pnr_dynamic_bullet_kernel(chain, obs_mode, obst) : explicit_kernels[chain][obs_mode][obst];
     int& resident = grids[device % PNR_MAX_DEVICES][stepping][chain][obs_mode][obst];
     if (resident == 0) {
-        cudaError_t e = cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PNR_DYN_SMEM);
+        cudaError_t e = pnr_prepare((const void*)kern, device, PNR_DYN_THREADS, PNR_DYN_SMEM, &resident);
         if (e != cudaSuccess) return e;
-        resident = pnr_dyn_resident((const void*)kern);
     }
     const int64_t per_cta = PNR_TILE_ENVS * PNR_DYN_WARPS;
     int64_t grid = (p.n_envs + per_cta - 1) / per_cta;
     if (grid > resident) grid = resident;
     if (grid < 1) grid = 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(PNR_DYN_THREADS); cfg.dynamicSmemBytes = PNR_DYN_SMEM; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pnr_pdl_enabled() ? 1 : 0;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kern, p, state, actions, obs, reward, done, stats, tick, domain, f_applied, f_delta, f_clip,
-                              multi);
+    return pnr_launch_pdl(kern, true, grid, PNR_DYN_THREADS, PNR_DYN_SMEM, stream, p, state, actions, obs, reward, done, stats,
+                          tick, domain, f_applied, f_delta, f_clip, multi);
 }

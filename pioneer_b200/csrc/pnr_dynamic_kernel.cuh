@@ -93,24 +93,20 @@ pnr_step_dynamic_kernel(const __grid_constant__ PnrParams p, float4* __restrict_
         const uint32_t tick_s = tick + (uint32_t)step;
 
         PnrPose o;
-        pnr_pose<true>(p, s, o);                               // q is inside the joint limits
-        bool reached = o.dist < p.done_distance;
-        if (fabsf(o.dist - p.done_distance) < p.done_band)
-            pnr_fk_tip_f64(p, s.r, s.tgt, o.ptr, o.dist, reached);
+        const bool reached = pnr_pose_reached<true>(p, s, o);   // q is inside the joint limits
         const float pot_new = pnr_potential(p, o.dist);
-        float rew = __fadd_rn(__fadd_rn(__fsub_rn(pot_new, s.pot), -p.penalty_step), reached ? p.award_done : 0.f);
+        float rew = pnr_reward(p, s.pot, pot_new, reached);
         if (OBSTACLES) {
             PnrSinCos sc;
 #pragma unroll
             for (int i = 0; i < PNR_DOF; ++i) { sc.sn[i] = o.sn[i]; sc.cs[i] = o.cs[i]; }
-            rew = __fsub_rn(rew, __fmul_rn(p.contact_penalty, pnr_contact_depth(p, sc, pnr_load_box(p, env), 0, 1)));
+            rew = pnr_contact_penalty(p, rew, pnr_contact_depth(p, sc, pnr_load_box(p, env), 0, 1));
         }
         s.pot = pot_new;
         s.t += 1;
         s.ep_ret = __fadd_rn(s.ep_ret, rew);
-        const bool timeout = p.max_episode_steps > 0 && s.t >= p.max_episode_steps;
-        const bool is_done = reached || timeout;
-        const uint8_t flags = (is_done ? PNR_DONE : 0) | ((timeout && !reached) ? PNR_TRUNCATED : 0);
+        bool is_done;
+        const uint8_t flags = pnr_step_flags(p, reached, s.t, is_done);
         if (active) {
             reward_s[env] = rew;
             done_s[env] = flags;
@@ -179,12 +175,13 @@ pnr_step_dynamic_kernel(const __grid_constant__ PnrParams p, float4* __restrict_
             }
             if (filt) {
                 __syncwarp();
-                double* f_slot = f_delta ? f_delta + (size_t)(blockIdx.x & (PNR_FILTER_SLOTS - 1)) * PNR_FILTER_DELTA_LEN : nullptr;
+                double* f_slot = f_delta ? pnr_filter_slot(f_delta, blockIdx.x) : nullptr;
 #pragma unroll 1
                 for (int pass = 0; pass < 4; ++pass) {
                     const int cc = pass * 32 + lane;                   // index among the 101 changing columns
                     if (cc < PNR_OBS_DIM - 36) {
                         const int c = cc < 18 ? cc : cc + 36;
+                        // pnr_filter_column written out: as a call it costs 4 to 16 bytes more spill in three instantiations
                         const float mean = f_applied[c], inv = f_applied[PNR_OBS_DIM + c];
                         float* colp = tile + c;
                         double s0 = 0.0, q0 = 0.0, s1 = 0.0, q1 = 0.0;
@@ -218,14 +215,7 @@ pnr_step_dynamic_kernel(const __grid_constant__ PnrParams p, float4* __restrict_
     }
     if (filt && f_delta && blockIdx.x == 0 && warp == 0) {         // rows pushed + the constant columns of all N rows
         if (lane == 0) atomicAdd(&f_delta[0], (double)N * multi.n_steps);
-        for (int c = 18 + lane; c < 54; c += 32) {
-            const int g = (c - 18) / PNR_DOF, j = (c - 18) % PNR_DOF;
-            const float x = g == 0 ? p.r_lo[j] : g == 1 ? p.cos_r_lo[j] : g == 2 ? p.sin_r_lo[j]
-                          : g == 3 ? p.r_hi[j] : g == 4 ? p.cos_r_hi[j] : p.sin_r_hi[j];
-            const double d = (double)(x - f_applied[c]);
-            atomicAdd(&f_delta[1 + c], (double)N * multi.n_steps * d);
-            atomicAdd(&f_delta[1 + PNR_OBS_DIM + c], (double)N * multi.n_steps * d * d);
-        }
+        for (int c = 18 + lane; c < 54; c += 32) pnr_filter_const_column(p, f_applied, f_delta, c, (double)N * multi.n_steps);
     }
     if (blockIdx.x == 0 && warp == 0 && lane == 0) atomicAdd(&stats->env_steps, (double)N * multi.n_steps);   // one writer per launch
     if (lane == 0) pnr_bulk_wait_read<0>();

@@ -112,7 +112,7 @@ pnr_filter_kernel(const float* __restrict__ in, float* __restrict__ out, int64_t
         }
         __syncthreads();                                        // the tile may be overwritten
     }
-    double* slot = delta + (size_t)(blockIdx.x & (PNR_FILTER_SLOTS - 1)) * PNR_FILTER_DELTA_LEN;
+    double* slot = pnr_filter_slot(delta, blockIdx.x);
     if (update && col_ok) {
         atomicAdd(&slot[1 + tid], acc_s);
         atomicAdd(&slot[1 + PNR_OBS_DIM + tid], acc_q);
@@ -251,27 +251,13 @@ pnr_iteration_sync_kernel(PnrStats* stats, int clear, double* filt_slots, double
     // 1. snapshot
     double v = 0.0;
     if (i < PNR_STATS_LEN) {
-        switch (i) {
-            case 0: v = stats->episodes; break;
-            case 1: v = stats->sum_return; break;
-            case 2: v = stats->sum_length; break;
-            case 3: v = stats->sum_return_sq; break;
-            case 4: v = (double)pnr_ordered_to_float(stats->max_return_ord); break;
-            case 5: v = (double)pnr_ordered_to_float(stats->min_return_ord); break;
-            case 6: v = stats->env_steps; break;
-            default: v = stats->reached; break;
-        }
+        v = pnr_stats_read(stats, i);
     } else if (i < len) {
         const int j = i - PNR_STATS_LEN;
         for (int k = 0; k < PNR_FILTER_SLOTS; ++k) v += filt_slots[(size_t)k * PNR_FILTER_DELTA_LEN + j];
     }
     __syncthreads();                                            // every field is read before the window is cleared
-    if (i == 0 && clear) {
-        stats->episodes = stats->sum_return = stats->sum_length = stats->sum_return_sq = stats->reached = 0.0;
-        stats->env_steps = 0.0;
-        stats->max_return_ord = pnr_float_to_ordered(-INFINITY);
-        stats->min_return_ord = pnr_float_to_ordered(INFINITY);
-    }
+    if (i == 0 && clear) pnr_stats_clear(stats);
     double acc = v;
     if (peers.world > 1) {
         unsigned char* mine = peers.window[peers.rank];
@@ -300,10 +286,8 @@ pnr_iteration_sync_kernel(PnrStats* stats, int clear, double* filt_slots, double
         if (i < len) {
             const double* sl = reinterpret_cast<const double*>(mine) + par * PNR_SYNC_MAX_PEERS * PNR_SYNC_SLOT_STRIDE + i;
             acc = pnr_ld_volatile_f64(sl);
-            for (int r = 1; r < peers.world; ++r) {
-                const double x = pnr_ld_volatile_f64(sl + (size_t)r * PNR_SYNC_SLOT_STRIDE);
-                acc = i == 4 ? fmax(acc, x) : (i == 5 ? fmin(acc, x) : acc + x);
-            }
+            for (int r = 1; r < peers.world; ++r)
+                acc = pnr_stats_combine(i, acc, pnr_ld_volatile_f64(sl + (size_t)r * PNR_SYNC_SLOT_STRIDE));
             if (!all_ok) acc = __longlong_as_double(0x7ff8000000000000ll);
         }
         if (i == 0) {
@@ -358,14 +342,8 @@ cudaError_t pnr_launch_filter(int device, const float* in, float* out, int64_t n
     static int resident[PNR_MAX_DEVICES] = {};
     int& res = resident[device % PNR_MAX_DEVICES];
     if (res == 0) {
-        cudaError_t e = cudaFuncSetAttribute((const void*)pnr_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             PNR_FILTER_TILE_BYTES);
+        cudaError_t e = pnr_prepare((const void*)pnr_filter_kernel, device, PNR_FILTER_THREADS, PNR_FILTER_TILE_BYTES, &res);
         if (e != cudaSuccess) return e;
-        int sms = 0, per_sm = 0;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)pnr_filter_kernel, PNR_FILTER_THREADS,
-                                                      PNR_FILTER_TILE_BYTES);
-        res = sms * (per_sm < 1 ? 1 : per_sm);
     }
     if (n_rows <= 0) return cudaSuccess;
     int64_t grid = (n_rows + PNR_FILTER_ROWS - 1) / PNR_FILTER_ROWS;

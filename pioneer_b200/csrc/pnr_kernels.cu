@@ -2,7 +2,6 @@
 // sm_100a; launched from pnr_api.cu.
 #include "pnr_kernels.cuh"
 #include "pnr_launch.h"
-#include <cstdlib>
 
 // ---------------------------------------------------------------------------------------------
 // K1: the fused env step.  One CTA of 4 warps owns a tile of 32 envs (lane = env); the work of ONE env is
@@ -68,29 +67,6 @@ __device__ __noinline__ float4 pnr_auto_reset(const PnrParams& p, float4* __rest
     return make_float4(tg[0], tg[1], tg[2], 0.f);
 }
 
-#ifdef PNR_TRACE
-// developer instrumentation (python -m pioneer_b200.build --trace): per-CTA phase timestamps of the first work items
-#define PNR_TRACE_SLOTS 12
-#define PNR_TRACE_CTAS 2048
-#define PNR_TRACE_ITERS 4
-__device__ unsigned long long pnr_trace_buf[PNR_TRACE_CTAS][2][PNR_TRACE_ITERS][PNR_TRACE_SLOTS];
-__device__ __forceinline__ void pnr_trace_mark(int part, int lane, int slot, int iter) {
-    if (lane == 0 && (part == 0 || part == 3) && blockIdx.x < PNR_TRACE_CTAS && iter < PNR_TRACE_ITERS) {
-        unsigned long long t;
-        if (slot == 0) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); else t = clock64();
-        pnr_trace_buf[blockIdx.x][part == 3][iter][slot] = t;
-    }
-}
-extern "C" int pnr_debug_trace(unsigned long long* out_host) {
-    return (int)cudaMemcpyFromSymbol(out_host, pnr_trace_buf, sizeof(pnr_trace_buf));
-}
-#define PNR_MARK(slot) pnr_trace_mark(part, lane, slot, trace_iter)
-#define PNR_TRACE_NEXT() (++trace_iter)
-#else
-#define PNR_MARK(slot)
-#define PNR_TRACE_NEXT()
-#endif
-
 // FILTER = true fuses the observation normaliser (pnr_filter.cu, 'ConcurrentMeanStdFilter') into the step: what leaves the
 // kernel is clip((x - mean) * inv_std), and the column statistics of the raw values go to the same float64 accumulator
 // pnr_filter_apply feeds, so the 548 B/env observation is never re-read.  Every warp normalises the columns it owns
@@ -128,10 +104,6 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
     // by one and run their set-up (constant columns, barriers) under this grid's tail; they stop at pnr_pdl_wait()
     pnr_pdl_trigger();
 
-#ifdef PNR_TRACE
-    int trace_iter = 0;
-#endif
-    PNR_MARK(0); PNR_MARK(1);
     const int j0 = part < 3 ? 2 * part : 0;                   // first joint of a joint warp
     float* rowj = row + j0;
     // loop-invariant limits of this warp's two joints, read once from the constant bank
@@ -204,7 +176,6 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
     pnr_pdl_wait();                                           // the previous step's state planes are complete and visible
     load_planes(t_idx);
     load_act(t_idx, 0);
-    PNR_MARK(2);
     int buf = 0;
     int64_t iter = 0;                                         // work items this CTA has started
     int32_t step = 0;                                         // step of the fragment (PnrMulti; 1 step for pnr_step)
@@ -243,9 +214,7 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
                 pnr_sincos_fast(r1[1], sn[1], cs[1]);
             };
             advance();
-            PNR_MARK(3);
             if (iter >= 1) pnr_bar_sync2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf);   // buffer reusable, resets published
-            PNR_MARK(4);
             if (step > 0 && ((s_reset >> lane) & 1u)) {       // the task warp reset this env after the previous step
                 st4 = make_float4(s_pub[j0 * 32 + lane], s_pub[(j0 + 1) * 32 + lane], 0.f, 0.f);
                 st2 = make_float2(0.f, 0.f);
@@ -259,11 +228,8 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             }
             pnr_bar_arrive2<PNR_BAR_HEAD, PNR_STEP_THREADS>(buf);
         } else {
-            PNR_MARK(3);
             pnr_bar_sync2<PNR_BAR_HEAD, PNR_STEP_THREADS>(buf);   // r, cos r, sin r of all six joints are in the tile
-            PNR_MARK(4);
         }
-        PNR_MARK(5);
 
         bool do_reset = false;
         // OBSTACLES: what the task warp carries across the DONE barrier (the penalty is summed from the joint warps' partials)
@@ -300,27 +266,7 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             }
             if (FILTER) {                                      // column pass over this warp's 30 changing columns
                 __syncwarp();
-                if (lane < 30) {
-                    float* colp = tile + f_col;
-                    double s1 = 0.0, q1 = 0.0;                 // second accumulator pair: two independent FP64 chains
-                    int r = 0;
-#pragma unroll 4
-                    for (; r + 1 < rows_valid; r += 2) {
-                        const float d0 = colp[r * PNR_OBS_DIM] - f_mean, d1 = colp[(r + 1) * PNR_OBS_DIM] - f_mean;
-                        const double e0 = (double)d0, e1 = (double)d1;
-                        f_sum += e0; f_sq = fma(e0, e0, f_sq);
-                        s1 += e1; q1 = fma(e1, e1, q1);
-                        colp[r * PNR_OBS_DIM] = fminf(fmaxf(d0 * f_inv, -f_clip), f_clip);
-                        colp[(r + 1) * PNR_OBS_DIM] = fminf(fmaxf(d1 * f_inv, -f_clip), f_clip);
-                    }
-                    if (r < rows_valid) {
-                        const float d0 = colp[r * PNR_OBS_DIM] - f_mean;
-                        const double e0 = (double)d0;
-                        f_sum += e0; f_sq = fma(e0, e0, f_sq);
-                        colp[r * PNR_OBS_DIM] = fminf(fmaxf(d0 * f_inv, -f_clip), f_clip);
-                    }
-                    f_sum += s1; f_sq += q1;
-                }
+                if (lane < 30) pnr_filter_column(tile + f_col, rows_valid, f_mean, f_inv, f_clip, f_sum, f_sq);
             }
         } else {
             // --- pose from the joint warps' sin/cos, distance, reward, done
@@ -347,13 +293,10 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
                 reached = bo.within != 0;
             }
             const float pot_new = pnr_potential(p, o.dist);
-            // (potential - old_potential) + (-penalty_step) + (award_done | 0), pioneer_knm_env.py:162-165
-            float rew = __fadd_rn(__fadd_rn(__fsub_rn(pot_new, pot_old), -p.penalty_step),
-                                  reached ? p.award_done : 0.f);
+            const float rew = pnr_reward(p, pot_old, pot_new, reached);
             t += 1;
-            const bool timeout = p.max_episode_steps > 0 && t >= p.max_episode_steps;
-            const bool is_done = reached || timeout;
-            const uint8_t flags = (is_done ? PNR_DONE : 0) | ((timeout && !reached) ? PNR_TRUNCATED : 0);
+            bool is_done;
+            const uint8_t flags = pnr_step_flags(p, reached, t, is_done);
             if (active) done_s[env] = flags;
             if (OBSTACLES) {                                   // the penalty arrives with DONE: reward, return and statistics wait
                 d_rew = rew; d_t = t; d_done = is_done; d_reached = reached;
@@ -389,17 +332,15 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             }
             do_reset = is_done && active && (p.auto_reset != 0);   // handled after DONE (rare)
         }
-        PNR_MARK(6);
         pnr_fence_async_smem();                               // generic-proxy tile writes -> async proxy
         if (part < 3) pnr_bar_arrive2<PNR_BAR_DONE, PNR_STEP_THREADS>(buf);
         else pnr_bar_sync2<PNR_BAR_DONE, PNR_STEP_THREADS>(buf);   // tile complete (joint planes stored after a last step)
-        PNR_MARK(7);
 
         if (part == 3) {
             if (OBSTACLES) {                                  // capsule penetration penalty, then the deferred writes
                 const float* pb = pen + buf * PNR_PEN_FLOATS + lane;
                 const float depth = (pb[0] + pb[32]) + pb[64];
-                const float rew = __fsub_rn(d_rew, __fmul_rn(p.contact_penalty, depth));
+                const float rew = pnr_contact_penalty(p, d_rew, depth);
                 st2.y = __fadd_rn(st2.y, rew);
                 if (active) {
                     reward_s[env] = rew;
@@ -444,8 +385,6 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
             __syncwarp();
             if (more) pnr_bar_arrive2<PNR_BAR_FREE, PNR_STEP_THREADS>(buf ^ 1);
         }
-        PNR_MARK(8);
-        PNR_TRACE_NEXT();
         if (!more) break;
         t_idx = next_tile;
         step = last ? 0 : step + 1;
@@ -457,20 +396,14 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
         if (FILTER) srow = scratch + buf * PNR_FSCRATCH_FLOATS + lane * PNR_FSCRATCH_STRIDE;
     }
     if (FILTER && f_delta != nullptr) {                       // column statistics of this CTA's rows, into copy blockIdx % SLOTS
-        double* f_slot = f_delta + (size_t)(blockIdx.x & (PNR_FILTER_SLOTS - 1)) * PNR_FILTER_DELTA_LEN;
+        double* f_slot = pnr_filter_slot(f_delta, blockIdx.x);
         if (part < 3) {
             if (lane < 30) {
                 atomicAdd(&f_slot[1 + f_col], f_sum);
                 atomicAdd(&f_slot[1 + PNR_OBS_DIM + f_col], f_sq);
             }
-            if (blockIdx.x == 0 && lane < 12) {                // the constant columns of all N rows, analytically
-                const int g = lane >> 1, j = j0 + (lane & 1), c = 18 + 6 * g + j;
-                const float x = g == 0 ? p.r_lo[j] : g == 1 ? p.cos_r_lo[j] : g == 2 ? p.sin_r_lo[j]
-                              : g == 3 ? p.r_hi[j] : g == 4 ? p.cos_r_hi[j] : p.sin_r_hi[j];
-                const double d = (double)(x - f_applied[c]);
-                atomicAdd(&f_delta[1 + c], (double)N * multi.n_steps * d);
-                atomicAdd(&f_delta[1 + PNR_OBS_DIM + c], (double)N * multi.n_steps * d * d);
-            }
+            if (blockIdx.x == 0 && lane < 12)                  // the constant columns of all N rows, analytically
+                pnr_filter_const_column(p, f_applied, f_delta, 18 + 6 * (lane >> 1) + j0 + (lane & 1), (double)N * multi.n_steps);
         } else {
 #pragma unroll
             for (int i = 0; i < 11; ++i) {
@@ -490,10 +423,6 @@ pnr_step_kernel(const __grid_constant__ PnrParams p, float4* __restrict__ state,
     }
     if (part == 3 && lane == 0 && blockIdx.x == 0) atomicAdd(&stats->env_steps, (double)N * multi.n_steps);   // one writer per launch
     if (part == 3 && lane == 0) pnr_bulk_wait_read<0>();      // smem must outlive the copy engine's reads
-#ifdef PNR_TRACE
-    trace_iter = 0;
-#endif
-    PNR_MARK(9);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -533,9 +462,7 @@ pnr_reset_observe_kernel(const __grid_constant__ PnrParams p, float4* __restrict
         if (obs_out) {
             // injected joint angles may lie anywhere: library sincos for every column here (not the hot path)
             PnrPose o;
-            pnr_pose<false>(p, s, o);
-            bool within;
-            if (fabsf(o.dist - p.done_distance) < p.done_band) pnr_fk_tip_f64(p, s.r, s.tgt, o.ptr, o.dist, within);
+            pnr_pose_reached<false>(p, s, o);
             if (tile_busy) pnr_tile_wait(lane);
             pnr_pack_obs_const(p, tile + lane * PNR_OBS_DIM);
             pnr_pack_obs_dyn<false>(p, tile + lane * PNR_OBS_DIM, s, o, s.pot);
@@ -569,33 +496,30 @@ __global__ void pnr_observe_done_kernel(const __grid_constant__ PnrParams p, flo
         PnrEnv s;
         pnr_load_env(state, N, env, s);
         PnrPose o;
-        pnr_pose<false>(p, s, o);
-        bool within;
-        if (fabsf(o.dist - p.done_distance) < p.done_band) pnr_fk_tip_f64(p, s.r, s.tgt, o.ptr, o.dist, within);
+        pnr_pose_reached<false>(p, s, o);
         pnr_pack_obs_const(p, row);
         pnr_pack_obs_dyn<false>(p, row, s, o, s.pot);
         if (f_applied) {
-            double* slot = f_delta ? f_delta + (size_t)(env & (PNR_FILTER_SLOTS - 1)) * PNR_FILTER_DELTA_LEN : nullptr;
+            double* slot = f_delta ? pnr_filter_slot(f_delta, (uint32_t)env) : nullptr;
             for (int c = 0; c < PNR_OBS_DIM; ++c) {
-                const float d = row[c] - f_applied[c];
                 if (slot) {
-                    atomicAdd(&slot[1 + c], (double)d);
-                    atomicAdd(&slot[1 + PNR_OBS_DIM + c], (double)d * (double)d);
+                    const double d = (double)(row[c] - f_applied[c]);
+                    atomicAdd(&slot[1 + c], d);
+                    atomicAdd(&slot[1 + PNR_OBS_DIM + c], d * d);
                 }
-                row[c] = fminf(fmaxf(d * f_applied[PNR_OBS_DIM + c], -f_clip), f_clip);
+                row[c] = pnr_normalise(row[c], f_applied[c], f_applied[PNR_OBS_DIM + c], f_clip);
             }
             if (slot) atomicAdd(&slot[0], 1.0);
         }
     }
 }
 
-cudaError_t pnr_launch_observe_done(const PnrParams& p, float4* state, const uint8_t* done, float* obs, float* terminal_out,
-                                    const float* f_applied, double* f_delta, float f_clip, cudaStream_t stream) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+cudaError_t pnr_launch_observe_done(const PnrParams& p, int device, float4* state, const uint8_t* done, float* obs,
+                                    float* terminal_out, const float* f_applied, double* f_delta, float f_clip,
+                                    cudaStream_t stream) {
+    const int64_t cap = (int64_t)pnr_sm_count(device) * 8;
     int64_t grid = (p.n_envs + 127) / 128;
-    if (grid > (int64_t)sms * 8) grid = (int64_t)sms * 8;
+    if (grid > cap) grid = cap;
     pnr_observe_done_kernel<<<(unsigned)grid, 128, 0, stream>>>(p, state, done, obs, terminal_out, f_applied, f_delta, f_clip);
     return cudaGetLastError();
 }
@@ -653,30 +577,20 @@ __global__ void pnr_compact_obs_kernel(const float* __restrict__ full, float* __
 
 __global__ void pnr_stats_snapshot_kernel(PnrStats* stats, double* out, int clear) {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
-        out[0] = stats->episodes; out[1] = stats->sum_return; out[2] = stats->sum_length;
-        out[3] = stats->sum_return_sq;
-        out[4] = (double)pnr_ordered_to_float(stats->max_return_ord);
-        out[5] = (double)pnr_ordered_to_float(stats->min_return_ord);
-        out[6] = stats->env_steps; out[7] = stats->reached;
-        if (clear) {
-            stats->episodes = stats->sum_return = stats->sum_length = stats->sum_return_sq = stats->reached = 0.0;
-            stats->env_steps = 0.0;
-            stats->max_return_ord = pnr_float_to_ordered(-INFINITY);
-            stats->min_return_ord = pnr_float_to_ordered(INFINITY);
-        }
+        for (int i = 0; i < PNR_STATS_LEN; ++i) out[i] = pnr_stats_read(stats, i);
+        if (clear) pnr_stats_clear(stats);
     }
 }
 
 // The reduction half of the path's one collective: `gathered` = the packed statistics vectors of all ranks (what one
-// all-gather delivered), out = SUM over {0,1,2,3,6,7}, MAX over 4, MIN over 5; `extra` doubles per rank behind the eight
-// (the observation filter's delta) are summed.  One small kernel instead of half a dozen indexing / reduction launches.
+// all-gather delivered), combined in rank order by pnr_stats_combine; `extra` doubles per rank behind the eight (the
+// observation filter's delta) are summed.  One small kernel instead of half a dozen indexing / reduction launches.
 __global__ void pnr_stats_merge_kernel(const double* __restrict__ gathered, int world, int len, double* __restrict__ out) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= len) return;
     double acc = gathered[c];
     for (int r = 1; r < world; ++r) {
-        const double x = gathered[(size_t)r * len + c];
-        acc = c == 4 ? fmax(acc, x) : (c == 5 ? fmin(acc, x) : acc + x);
+        acc = pnr_stats_combine(c, acc, gathered[(size_t)r * len + c]);
     }
     out[c] = acc;
 }
@@ -689,28 +603,26 @@ cudaError_t pnr_launch_stats_merge(const double* gathered, int world, int len, d
 // ---------------------------------------------------------------------------------------------
 // host-callable launchers (declared in pnr_launch.h)
 // ---------------------------------------------------------------------------------------------
-// developer knob: PNR_NO_PDL=1 launches the step kernels without programmatic dependent launch (A/B measurements)
-bool pnr_pdl_enabled() {
-    static const bool on = getenv("PNR_NO_PDL") == nullptr;
-    return on;
+int pnr_sm_count(int device) {
+    static int sms_of[PNR_MAX_DEVICES] = {};
+    int& sms = sms_of[device % PNR_MAX_DEVICES];
+    if (sms == 0) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    return sms;
 }
 
-static int pnr_resident_grid(const void* fn, size_t smem) {
-    int dev = 0, sms = 0, per_sm = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PNR_STEP_THREADS, smem);
-    if (per_sm < 1) per_sm = 1;
-    return sms * per_sm;
-}
-
-template <typename K>
-static cudaError_t pnr_prepare(K kernel, size_t smem, int* grid_out) {
-    cudaError_t e = cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+cudaError_t pnr_prepare(const void* kernel, int device, int threads, size_t smem, int* resident) {
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    *grid_out = pnr_resident_grid((const void*)kernel, smem);
+    int per_sm = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
+    *resident = pnr_sm_count(device) * (per_sm < 1 ? 1 : per_sm);
     return cudaSuccess;
 }
+
+// Resident CTAs per SM of the kinematic step kernel, measured on B200 (profiles/r03_step_65536.md): with the steps of a
+// fragment pipelined per tile, 4 CTAs per SM stream best from 2,048 tiles on (131,072 envs: 14.2 us per step against 15.1
+// with 5 or 6; 65,536 envs: 7.9 against 8.2 with 6); smaller grids keep 6 per SM so that up to 888 tiles run at once.
+static int pnr_step_ctas_per_sm(int64_t n_tiles) { return n_tiles >= 2048 ? 4 : 6; }
 
 // grid = min(CTAs needed, CTAs resident on the whole GPU): a multiple of the SM count once the batch is large
 static int64_t pnr_grid_for(int64_t n_envs, int envs_per_cta, int resident) {
@@ -740,30 +652,17 @@ cudaError_t pnr_launch_step(const PnrParams& p, int device, int arith, int obs_m
     const size_t smem = (filt ? PNR_STEP_SMEM_FILTER : PNR_STEP_SMEM) + (obst ? PNR_STEP_SMEM_OBST : 0);
     int& resident = grids[device % PNR_MAX_DEVICES][arith][obs_mode][obst][filt];
     if (resident == 0) {
-        cudaError_t e = pnr_prepare(k, smem, &resident);
+        cudaError_t e = pnr_prepare((const void*)k, device, PNR_STEP_THREADS, smem, &resident);
         if (e != cudaSuccess) return e;
     }
-    // Resident CTAs per SM, measured on B200 (profiles/r03_step_65536.md): with the steps of a fragment pipelined per tile,
-    // 4 CTAs per SM stream best from 2,048 tiles on (131,072 envs: 14.2 us per step against 15.1 with 5 or 6; 65,536 envs:
-    // 7.9 against 8.2 with 6); smaller grids keep 6 per SM so that up to 888 tiles run at once.
-    static int sms_of[PNR_MAX_DEVICES] = {};
-    int& dev_sms = sms_of[device % PNR_MAX_DEVICES];
-    if (dev_sms == 0) cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, device);
     const int64_t n_tiles = (p.n_envs + PNR_TILE_ENVS - 1) / PNR_TILE_ENVS;
-    int per_sm = n_tiles >= 2048 ? 4 : 6;
-    if (const char* e = getenv("PNR_CTAS_PER_SM")) per_sm = atoi(e) > 0 ? atoi(e) : per_sm;   // developer knob
-    int cap = per_sm * dev_sms < resident ? per_sm * dev_sms : resident;
-    const int64_t grid = pnr_grid_for(p.n_envs, PNR_TILE_ENVS, cap);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(PNR_STEP_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    const int cap = pnr_step_ctas_per_sm(n_tiles) * pnr_sm_count(device);
+    const int64_t grid = pnr_grid_for(p.n_envs, PNR_TILE_ENVS, cap < resident ? cap : resident);
     // programmatic dependent launch pays where the launch tail is a visible share of the step (65,536 envs: 13.2 -> 11.8 us);
     // on long grids the early-resident successor only takes SM slots from this grid (1,048,576 envs: 146 -> 151 us).
     // One launch per fragment: fragments are timed the same with and without it (profiles/r03_step_65536.md)
-    attr[0].val.programmaticStreamSerializationAllowed = (pnr_pdl_enabled() && n_tiles <= 8192) ? 1 : 0;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, k, p, state, actions, obs, reward, done, stats, tick, domain, f_applied, f_delta, f_clip, multi);
+    return pnr_launch_pdl(k, n_tiles <= 8192, grid, PNR_STEP_THREADS, smem, stream, p, state, actions, obs, reward, done,
+                          stats, tick, domain, f_applied, f_delta, f_clip, multi);
 }
 
 cudaError_t pnr_launch_reset_observe(const PnrParams& p, int device, int mode, float4* state, const int64_t* idx, int64_t n,
@@ -774,7 +673,7 @@ cudaError_t pnr_launch_reset_observe(const PnrParams& p, int device, int mode, f
     static int grids[PNR_MAX_DEVICES][2] = {};
     int& resident = grids[device % PNR_MAX_DEVICES][mode];
     if (resident == 0) {
-        cudaError_t e = pnr_prepare(kernels[mode], PNR_RO_SMEM, &resident);
+        cudaError_t e = pnr_prepare((const void*)kernels[mode], device, PNR_STEP_THREADS, PNR_RO_SMEM, &resident);
         if (e != cudaSuccess) return e;
     }
     if (n <= 0) return cudaSuccess;
@@ -800,14 +699,12 @@ cudaError_t pnr_launch_box_io(bool set, float4* box_a, float* box_z, int64_t N, 
     return cudaGetLastError();
 }
 
-cudaError_t pnr_launch_compact_obs(const float* full, float* compact, int64_t n_rows, cudaStream_t stream) {
+cudaError_t pnr_launch_compact_obs(int device, const float* full, float* compact, int64_t n_rows, cudaStream_t stream) {
     const int64_t n_out = n_rows * PNR_OBS_COMPACT_DIM;
     if (n_out <= 0) return cudaSuccess;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int64_t cap = (int64_t)pnr_sm_count(device) * 8;           // 8 CTAs of 256 threads per SM, grid-stride
     int64_t grid = (n_out + 255) / 256;
-    if (grid > (int64_t)sms * 8) grid = (int64_t)sms * 8;          // 8 CTAs of 256 threads per SM, grid-stride
+    if (grid > cap) grid = cap;
     pnr_compact_obs_kernel<<<(unsigned)grid, 256, 0, stream>>>(full, compact, n_out);
     return cudaGetLastError();
 }

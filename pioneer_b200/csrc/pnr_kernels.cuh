@@ -484,6 +484,32 @@ __device__ __forceinline__ float pnr_potential(const PnrParams& p, float dist) {
     return __fdiv_rn(p.pot_max, __fadd_rn(__fdiv_rn(dist, p.pot_slope), 1.f));
 }
 
+// The step kernels' task code, written once so that every mode rounds alike.
+// Reward (pioneer_knm_env.py:162-165, in this rounding order): (potential - old_potential) + (-penalty_step) + (award_done | 0)
+__device__ __forceinline__ float pnr_reward(const PnrParams& p, float pot_old, float pot_new, bool reached) {
+    return __fadd_rn(__fadd_rn(__fsub_rn(pot_new, pot_old), -p.penalty_step), reached ? p.award_done : 0.f);
+}
+// done / TimeLimit flags after the episode's t-th step: TRUNCATED marks a timeout that did not also reach the target
+__device__ __forceinline__ uint8_t pnr_step_flags(const PnrParams& p, bool reached, int32_t t, bool& is_done) {
+    const bool timeout = p.max_episode_steps > 0 && t >= p.max_episode_steps;
+    is_done = reached || timeout;
+    return (is_done ? PNR_DONE : 0) | ((timeout && !reached) ? PNR_TRUNCATED : 0);
+}
+// obstacle variant: the reward less the capsule penetration penalty
+__device__ __forceinline__ float pnr_contact_penalty(const PnrParams& p, float rew, float depth) {
+    return __fsub_rn(rew, __fmul_rn(p.contact_penalty, depth));
+}
+
+// pose of the env's current r and whether it reached its target, decided in float64 where float32 could flip it
+// (thread-per-env kernels; the step kernel's task warp takes the sin / cos of its joint warps from shared memory)
+template <bool FAST>
+__device__ __forceinline__ bool pnr_pose_reached(const PnrParams& p, const PnrEnv& s, PnrPose& o) {
+    pnr_pose<FAST>(p, s, o);
+    bool reached = o.dist < p.done_distance;
+    if (fabsf(o.dist - p.done_distance) < p.done_band) pnr_fk_tip_f64(p, s.r, s.tgt, o.ptr, o.dist, reached);
+    return reached;
+}
+
 // ---------------------------------------------------------------------------------------------
 // observe() (pioneer_knm_env.py:184-211): the 137-float row of one env, written into the warp's
 // shared-memory tile at row `lane`.  The 36 columns that never change (r_lo, r_hi and their cos / sin,
@@ -550,6 +576,42 @@ __device__ __forceinline__ void pnr_pack_obs_dyn(const PnrParams& p, float* __re
 // the observation normaliser's element map: clip((x - mean) * inv_std, +-clip)   (pnr_filter.cu, fused step kernel)
 __device__ __forceinline__ float pnr_normalise(float x, float mean, float inv_std, float clip) {
     return fminf(fmaxf((x - mean) * inv_std, -clip), clip);
+}
+
+// The fused normaliser's column pass: one column of a shared-memory tile (`rows` rows) is normalised in place, and the
+// float64 sum and sum of squares of x - mean are ADDED to s and q.  Two independent chains; the statistics depend on the
+// order of these additions.
+__device__ __forceinline__ void pnr_filter_column(float* colp, int rows, float mean, float inv, float clip, double& s,
+                                                  double& q) {
+    double s1 = 0.0, q1 = 0.0;
+    int r = 0;
+#pragma unroll 4
+    for (; r + 1 < rows; r += 2) {
+        const float d0 = colp[r * PNR_OBS_DIM] - mean, d1 = colp[(r + 1) * PNR_OBS_DIM] - mean;
+        const double e0 = (double)d0, e1 = (double)d1;
+        s += e0; q = fma(e0, e0, q);
+        s1 += e1; q1 = fma(e1, e1, q1);
+        colp[r * PNR_OBS_DIM] = fminf(fmaxf(d0 * inv, -clip), clip);
+        colp[(r + 1) * PNR_OBS_DIM] = fminf(fmaxf(d1 * inv, -clip), clip);
+    }
+    if (r < rows) {
+        const float d0 = colp[r * PNR_OBS_DIM] - mean;
+        const double e0 = (double)d0;
+        s += e0; q = fma(e0, e0, q);
+        colp[r * PNR_OBS_DIM] = fminf(fmaxf(d0 * inv, -clip), clip);
+    }
+    s += s1; q += q1;
+}
+
+// the statistics of constant column c (18 <= c < 54) over `rows` rows, added analytically to the accumulator
+__device__ __forceinline__ void pnr_filter_const_column(const PnrParams& p, const float* __restrict__ f_applied,
+                                                        double* __restrict__ f_delta, int c, double rows) {
+    const int g = (c - 18) / PNR_DOF, j = (c - 18) % PNR_DOF;
+    const float x = g == 0 ? p.r_lo[j] : g == 1 ? p.cos_r_lo[j] : g == 2 ? p.sin_r_lo[j]
+                  : g == 3 ? p.r_hi[j] : g == 4 ? p.cos_r_hi[j] : p.sin_r_hi[j];
+    const double d = (double)(x - f_applied[c]);
+    atomicAdd(&f_delta[1 + c], rows * d);
+    atomicAdd(&f_delta[1 + PNR_OBS_DIM + c], rows * d * d);
 }
 
 // ---- per-joint column groups for the step kernel's joint warps (joint j owns columns j, 6+j, ..., 120+j) ----

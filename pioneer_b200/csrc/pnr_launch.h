@@ -1,6 +1,7 @@
 // Host-side launch interface between pnr_api.cu (C-ABI) and the kernel translation units.
 #pragma once
 #include <cuda_runtime.h>
+#include <utility>
 #include "pnr_device.cuh"
 
 #define PNR_STEP_WARPS 4
@@ -29,6 +30,28 @@
 // each of 274 addresses and the kernel's tail took 13 us (tools/fuse_probe.py: 18.5 us without statistics, 31.7 us with).
 // pnr_launch_filter_fold adds copies 1.. into copy 0 (what the host and the all-reduce read) and clears them.
 #define PNR_FILTER_SLOTS 64
+__device__ __forceinline__ double* pnr_filter_slot(double* delta, uint32_t i) {
+    return delta + (size_t)(i & (PNR_FILTER_SLOTS - 1)) * PNR_FILTER_DELTA_LEN;
+}
+
+// the SM count of `device`, queried once
+int pnr_sm_count(int device);
+// once per kernel and device: allow `smem` bytes of dynamic shared memory and count the CTAs of `threads` threads the whole
+// GPU holds at once (at least one per SM)
+cudaError_t pnr_prepare(const void* kernel, int device, int threads, size_t smem, int* resident);
+
+// Launch with programmatic dependent launch on or off (pnr_pdl_wait / pnr_pdl_trigger in pnr_device.cuh)
+template <typename Kern, typename... Args>
+inline cudaError_t pnr_launch_pdl(Kern kernel, bool pdl, int64_t grid, int threads, size_t smem, cudaStream_t stream,
+                                  Args&&... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
 
 // f_applied != NULL selects the fused normaliser (kinematic: a separate instantiation, float32 arithmetic and terminal
 // observations only; dynamic: a run-time switch, both observation modes); f_delta may be NULL (normalise, no statistics)
@@ -43,11 +66,11 @@ cudaError_t pnr_launch_reset_observe(const PnrParams& p, int device, int mode, f
                                      cudaStream_t stream);
 cudaError_t pnr_launch_state_io(bool set, float4* state, int64_t N, float* r, float* v, float* a, float* potential,
                                 float* target, int32_t* t, float* ep_return, cudaStream_t stream);
-bool pnr_pdl_enabled();
-cudaError_t pnr_launch_observe_done(const PnrParams& p, float4* state, const uint8_t* done, float* obs, float* terminal_out,
-                                    const float* f_applied, double* f_delta, float f_clip, cudaStream_t stream);
+cudaError_t pnr_launch_observe_done(const PnrParams& p, int device, float4* state, const uint8_t* done, float* obs,
+                                    float* terminal_out, const float* f_applied, double* f_delta, float f_clip,
+                                    cudaStream_t stream);
 cudaError_t pnr_launch_box_io(bool set, float4* box_a, float* box_z, int64_t N, float* box, cudaStream_t stream);
-cudaError_t pnr_launch_compact_obs(const float* full, float* compact, int64_t n_rows, cudaStream_t stream);
+cudaError_t pnr_launch_compact_obs(int device, const float* full, float* compact, int64_t n_rows, cudaStream_t stream);
 cudaError_t pnr_launch_tick_advance(PnrStats* stats, uint32_t n, int absolute, cudaStream_t stream);
 cudaError_t pnr_launch_env_steps_set(PnrStats* stats, double env_steps, cudaStream_t stream);
 cudaError_t pnr_launch_stats_merge(const double* gathered, int world, int len, double* out, cudaStream_t stream);

@@ -15,9 +15,6 @@ import torch.distributed as dist
 
 from .batched_env import STATS_FIELDS
 
-SUM_SLOTS = (0, 1, 2, 3, 6, 7)
-MAX_SLOTS = (4, 5)
-
 
 def bind_to_gpu_numa_node(device_index: int) -> Optional[int]:
     """Pin this process to the CPUs of the NUMA node the GPU hangs off, BEFORE any pinned host buffer is allocated, so

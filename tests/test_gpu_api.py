@@ -239,6 +239,21 @@ def test_step_many_equals_stepping(mode, n):
         for t in range(T):
             o, r, f = b.step_tensor(actions[t])
             assert torch.equal(f, flg[t]) and torch.equal(r, rew[t]) and torch.equal(o, obs[t]), (call, t)
+    # T = 0 launches nothing; T = 1 reads no stride, so strides that are no multiple of 16 (obs) or 8 (actions) bytes pass
+    from pioneer_b200 import _cabi
+    launches = a.launch_count
+    _cabi.check(a._lib.pnr_step_many(a._h, 0, actions.data_ptr(), 1, obs.data_ptr(), 1, rew.data_ptr(), flg.data_ptr(),
+                                     a._stream()), "pnr_step_many")
+    assert a.launch_count == launches
+    act1 = torch.zeros(n * 6 + 1, device="cuda").as_strided((1, n, 6), (n * 6 + 1, 6, 1))      # view() would reset stride(0)
+    obs1 = torch.zeros(n * 137 + 1, device="cuda").as_strided((1, n, 137), (n * 137 + 1, 137, 1))
+    act1[0] = lo + torch.rand((n, 6), device="cuda", generator=g) * (hi - lo)
+    rew1, flg1 = torch.zeros((1, n), device="cuda"), torch.zeros((1, n), dtype=torch.uint8, device="cuda")
+    assert act1.stride(0) * 4 % 8 and obs1.stride(0) * 4 % 16
+    a.step_many(act1, obs1, rew1, flg1)
+    assert a.launch_count == launches + 1
+    o, r, f = b.step_tensor(act1[0])
+    assert torch.equal(f, flg1[0]) and torch.equal(r, rew1[0]) and torch.equal(o, obs1[0])
     sa, sb = a.state(), b.state()
     assert all(torch.equal(sa[k], sb[k]) for k in sa)
     assert a.episode_stats() == b.episode_stats()
