@@ -6,6 +6,7 @@ import pytest
 
 torch = pytest.importorskip("torch")
 
+from tests._gpu import dynamic_env, fragments_equal_single_steps, kinematic_env, uniform_actions
 from tests._util import golden_case, load_golden
 
 pytestmark = pytest.mark.gpu
@@ -222,33 +223,21 @@ def test_step_many_equals_stepping(mode, n):
     """pnr_step_many gives bit for bit what T separate pnr_step calls give, call after call.  The fragment is ONE launch:
     every CTA (kinematic mode; a CTA barrier between the steps) or warp (dynamic mode; env state in registers) runs the T
     steps on its own tiles -- incl. ragged last tiles, several tiles per CTA / warp, auto-resets between the steps."""
-    from pioneer_b200 import BatchConfig, BatchedPioneerEnv, SimulationConfig
-    kw = dict(seed=4, simulation_config=SimulationConfig(gravity=9.81 if mode == "dynamic" else 0.0),
-              batch_config=BatchConfig(mode=mode, kp=2000.0, kd=500.0, torque_scale=1e5, max_episode_steps=5))
-    a, b = BatchedPioneerEnv(n, **kw), BatchedPioneerEnv(n, **kw)
-    T = 7 if n < 200000 else 3
-    g = torch.Generator(device="cuda").manual_seed(0)
-    lo, hi = torch.as_tensor(a.action_space.low).cuda(), torch.as_tensor(a.action_space.high).cuda()
-    n_pad = (n + 3) // 4 * 4
-    for call in range(4 if n < 200000 else 2):
-        actions = lo + torch.rand((T, n, 6), device="cuda", generator=g) * (hi - lo)
-        obs = torch.zeros((T, n_pad, 137), device="cuda")[:, :n]
-        rew = torch.zeros((T, n), device="cuda")
-        flg = torch.zeros((T, n), dtype=torch.uint8, device="cuda")
-        a.step_many(actions, obs, rew, flg)
-        for t in range(T):
-            o, r, f = b.step_tensor(actions[t])
-            assert torch.equal(f, flg[t]) and torch.equal(r, rew[t]) and torch.equal(o, obs[t]), (call, t)
-    # T = 0 launches nothing; T = 1 reads no stride, so strides that are no multiple of 16 (obs) or 8 (actions) bytes pass
     from pioneer_b200 import _cabi
-    launches = a.launch_count
-    _cabi.check(a._lib.pnr_step_many(a._h, 0, actions.data_ptr(), 1, obs.data_ptr(), 1, rew.data_ptr(), flg.data_ptr(),
-                                     a._stream()), "pnr_step_many")
-    assert a.launch_count == launches
+    make = kinematic_env if mode == "kinematic" else dynamic_env
+    a, b = make(n, max_episode_steps=5, seed=4), make(n, max_episode_steps=5, seed=4)
+    g = torch.Generator(device="cuda").manual_seed(0)
+    fragments_equal_single_steps(a, b, T=7 if n < 200000 else 3, fragments=4 if n < 200000 else 2, generator=g,
+                                 return_rtol=0)
+    # T = 0 launches nothing; T = 1 reads no stride, so strides that are no multiple of 16 (obs) or 8 (actions) bytes pass
     act1 = torch.zeros(n * 6 + 1, device="cuda").as_strided((1, n, 6), (n * 6 + 1, 6, 1))      # view() would reset stride(0)
     obs1 = torch.zeros(n * 137 + 1, device="cuda").as_strided((1, n, 137), (n * 137 + 1, 137, 1))
-    act1[0] = lo + torch.rand((n, 6), device="cuda", generator=g) * (hi - lo)
     rew1, flg1 = torch.zeros((1, n), device="cuda"), torch.zeros((1, n), dtype=torch.uint8, device="cuda")
+    launches = a.launch_count
+    _cabi.check(a._lib.pnr_step_many(a._h, 0, act1.data_ptr(), 1, obs1.data_ptr(), 1, rew1.data_ptr(), flg1.data_ptr(),
+                                     a._stream()), "pnr_step_many")
+    assert a.launch_count == launches
+    act1[0] = uniform_actions(a, g, 1)[0]
     assert act1.stride(0) * 4 % 8 and obs1.stride(0) * 4 % 16
     a.step_many(act1, obs1, rew1, flg1)
     assert a.launch_count == launches + 1

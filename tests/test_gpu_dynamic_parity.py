@@ -21,128 +21,16 @@ import pytest
 
 torch = pytest.importorskip("torch")
 
-from oracle.c_dyn_oracle import CDynOracleBatch, DynEnvConfig
+from tests._gpu import BULLET_BARS, c_dyn_oracle_for, dynamic_env, host_boxes, lockstep, setpoints
 
 pytestmark = pytest.mark.gpu
-
-PD = dict(gravity=9.81, kp=2000.0, kd=500.0, torque_scale=1e5)          # bench.py's dynamic-mode workload
-
-
-def make(n, obs_mode="terminal", limit=500, obstacles=(), penalty=0.0, random_box=False, seed=0, env_id_base=0, bullet=None,
-         **dyn):
-    from pioneer_b200 import BatchConfig, BatchedPioneerEnv, SimulationConfig
-    bc = BatchConfig(mode="dynamic", kp=dyn.get("kp", 0.0), kd=dyn.get("kd", 0.0), torque_scale=dyn.get("torque_scale", 1.0),
-                     max_episode_steps=limit, auto_reset=True, obs_mode=obs_mode, obstacles=list(obstacles),
-                     contact_penalty=penalty, random_box=random_box, **({"stepping": "bullet", **bullet} if bullet else {}))
-    env = BatchedPioneerEnv(n, batch_config=bc, simulation_config=SimulationConfig(gravity=dyn.get("gravity", 0.0)), seed=seed,
-                            env_id_base=env_id_base)
-    cfg = DynEnvConfig(gravity=dyn.get("gravity", 0.0), kp=bc.kp, kd=bc.kd, torque_scale=bc.torque_scale,
-                       max_episode_steps=limit, obstacles=tuple((o.kind, o.position, o.extent) for o in obstacles),
-                       contact_penalty=penalty, **({"stepping": "bullet", **bullet} if bullet else {}),
-                       random_box=(bc.box_pos_lo, bc.box_pos_hi, bc.box_size_lo, bc.box_size_hi) if random_box else None)
-    orc = CDynOracleBatch(env.chain, n, cfg, env_id_base=env_id_base, seed=seed, obs_mode=obs_mode)
-    return env, orc
-
-
-def check_obs(obs, o_obs, worst):
-    """obs: device float32 [n,137]; o_obs: oracle float64 computed from the SAME float32 (q, qd, a)."""
-    d = np.abs(obs.astype(np.float64) - o_obs)
-    for cols in (slice(0, 6), slice(90, 96), slice(108, 114), slice(18, 24), slice(36, 42), slice(129, 132)):
-        assert not d[:, cols].any(), f"value columns {cols} must be bit-exact"
-    worst["trig"] = max(worst.get("trig", 0.0), float(d[:, 6:90].max()), float(d[:, 96:108].max()), float(d[:, 114:126].max()))
-    worst["ptr"] = max(worst.get("ptr", 0.0), float(d[:, 126:129].max()), float(d[:, 132:136].max()))
-    worst["pot"] = max(worst.get("pot", 0.0), float(d[:, 136].max()))
-
-
-def lockstep(env, orc, steps, action_fn, obs_mode="terminal", check_every=1, bars=(5e-6, 5e-7, 5e-5, 5e-6)):
-    n = env.n_envs
-    s0, o0 = env.state(), orc.state()
-    assert np.array_equal(s0["r"].cpu().numpy().astype(np.float64), o0["q"])         # same Philox reset draws
-    assert np.array_equal(s0["target"].cpu().numpy().astype(np.float64), o0["target"])
-    worst = {}
-    n_done = pairs = free_pairs = 0
-    for t in range(steps):
-        act = action_fn(t)
-        obs, reward, flags = env.step_tensor(torch.as_tensor(act).cuda())
-        obs, reward, flags = obs.cpu().numpy(), reward.cpu().numpy(), flags.cpu().numpy()
-        if obs_mode == "terminal":
-            q32, qd32, mask = obs[:, 0:6], obs[:, 90:96], None                        # the post-substep state of EVERY env
-        else:                                                                         # finished rows show the next episode
-            mask = (flags & 1) == 0
-            st = env.state()
-            q32, qd32 = st["r"].cpu().numpy(), st["v"].cpu().numpy()
-        out = orc.step(act, adopt=(q32, qd32, None if mask is None else mask.astype(np.uint8)), want_obs=(t % check_every == 0))
-        # ---- the dynamics: where float64 arrives from the same float32 start.  An inelastic joint stop is a discontinuity
-        # (qd := 0): an env in which either side ran into a stop during this step may legitimately differ by qd * dt, so the
-        # bars apply to the envs that stayed clear of the stops on both sides; the others are counted
-        at_stop = ((q32 <= env.r_lo) | (q32 >= env.r_hi)).any(axis=1)
-        free = (out["touched"] == 0) & ~at_stop
-        if mask is not None:
-            free &= mask
-        pairs += int(n if mask is None else mask.sum())
-        free_pairs += int(free.sum())
-        dq = np.abs(q32.astype(np.float64) - out["own_q"])[free]
-        dqd = np.abs(qd32.astype(np.float64) - out["own_qd"])[free]
-        if dq.size:
-            bar_q = bars[0] + bars[1] * np.abs(out["own_q"][free])
-            bar_qd = bars[2] + bars[3] * np.abs(out["own_qd"][free])
-            if not (dq <= bar_q).all() or not (dqd <= bar_qd).all():
-                i, j = np.unravel_index(np.argmax(dq / bar_q), dq.shape)
-                i2, j2 = np.unravel_index(np.argmax(dqd / bar_qd), dqd.shape)
-                rows = np.nonzero(free)[0]
-                raise AssertionError(f"step {t}: dq {dq[i, j]:.3e} (bar {bar_q[i, j]:.3e}) env {rows[i]} joint {j} qd "
-                                     f"{out['own_qd'][rows[i]]}; dqd {dqd[i2, j2]:.3e} (bar {bar_qd[i2, j2]:.3e}) env {rows[i2]} "
-                                     f"joint {j2} qd {out['own_qd'][rows[i2]]} q {out['own_q'][rows[i2]]} act {act[rows[i2]]}")
-            worst["dq"] = max(worst.get("dq", 0.0), float(dq.max()))
-            worst["dqd"] = max(worst.get("dqd", 0.0), float(dqd.max()))
-            worst["qd_abs"] = max(worst.get("qd_abs", 0.0), float(np.abs(out["own_qd"][free]).max()))
-        # ---- the env layer on identical inputs
-        assert np.array_equal(flags, out["flags"]), (t, int((flags != out["flags"]).sum()))
-        dr = np.abs(reward.astype(np.float64) - out["reward"])
-        if mask is not None:
-            dr = dr[mask]                                                             # finished rows: the oracle used its own q
-        if dr.size:
-            assert dr.max() <= 2e-3, (t, float(dr.max()))
-            worst["reward"] = max(worst.get("reward", 0.0), float(dr.max()))
-        if out["obs"] is not None:
-            check_obs(obs, out["obs"], worst)
-        n_done += int((flags & 1).sum())
-    assert worst.get("trig", 0.0) <= 1e-6 and worst.get("ptr", 0.0) <= 2e-4 and worst.get("pot", 0.0) <= 1e-3, worst
-    worst["free_fraction"] = free_pairs / max(pairs, 1)
-    # ---- after the run: the reset envs carry the oracle's Philox draws, counters and statistics agree
-    s, o = env.state(), orc.state()
-    assert np.array_equal(s["t"].cpu().numpy(), o["t"])
-    assert np.array_equal(s["target"].cpu().numpy().astype(np.float64), o["target"])
-    assert np.array_equal(s["r"].cpu().numpy().astype(np.float64), o["q"])            # adopted or freshly reset: identical
-    assert np.abs(s["potential"].cpu().numpy() - o["potential"]).max() <= 1e-3
-    assert np.abs(s["ep_return"].cpu().numpy() - o["ep_return"]).max() <= 5e-2
-    st, os_ = env.episode_stats(), orc.stats
-    assert st["episodes"] == os_[0] == n_done and st["sum_length"] == os_[2] and st["env_steps"] == os_[6] == steps * n
-    assert st["reached_target"] == os_[7]
-    if n_done:
-        assert abs(st["sum_return"] - os_[1]) <= 5e-2 * n_done and abs(st["max_return"] - os_[4]) <= 5e-2
-        assert abs(st["min_return"] - os_[5]) <= 5e-2
-    return worst, n_done
-
-
-def setpoints(env, seed, hold=25):
-    """New PD set points every `hold` steps (uniform in the joint range): long transients, joints driven into the stops."""
-    rng = np.random.default_rng(seed)
-    cache = {}
-
-    def fn(t):
-        k = t // hold
-        if k not in cache:
-            cache.clear()
-            cache[k] = rng.uniform(env.r_lo, env.r_hi, size=(env.n_envs, 6)).astype(np.float32)
-        return cache[k]
-    return fn
 
 
 def test_config3_65536_envs_pd_control_timelimit_autoreset():
     """BASELINE.json configs[2]: 65,536 envs, joint limits, PD position control, TimeLimit + in-kernel auto-reset; 200 steps
     with TimeLimit 64 => every env goes through three episode ends and Philox resets."""
-    env, orc = make(65536, limit=64, seed=12, **PD)
+    env = dynamic_env(65536, max_episode_steps=64, seed=12)
+    orc = c_dyn_oracle_for(env, 12)
     worst, n_done = lockstep(env, orc, 200, setpoints(env, 1), check_every=10)
     assert n_done >= 3 * 65536 and worst["free_fraction"] > 0.85
     print("config3 dynamic parity, worst:", worst)
@@ -150,7 +38,8 @@ def test_config3_65536_envs_pd_control_timelimit_autoreset():
 
 
 def test_autoreset_observation_mode_at_16384_envs():
-    env, orc = make(16384, obs_mode="autoreset", limit=40, seed=5, env_id_base=1 << 33, **PD)
+    env = dynamic_env(16384, obs_mode="autoreset", max_episode_steps=40, seed=5, env_id_base=1 << 33)
+    orc = c_dyn_oracle_for(env, 5)
     worst, n_done = lockstep(env, orc, 100, setpoints(env, 2), obs_mode="autoreset", check_every=5)
     assert n_done >= 2 * 16384 and worst["free_fraction"] > 0.85   # (+ the rare env that reaches its target)
     print("autoreset mode, worst:", worst)
@@ -159,7 +48,8 @@ def test_autoreset_observation_mode_at_16384_envs():
 
 def test_torque_control_with_gravity():
     n = 8192
-    env, orc = make(n, limit=30, seed=3, gravity=9.81, torque_scale=40.0)
+    env = dynamic_env(n, control="torque", gravity=9.81, torque_scale=40.0, max_episode_steps=30, seed=3)
+    orc = c_dyn_oracle_for(env, 3)
     rng = np.random.default_rng(4)
     tau_max = (np.asarray(env.chain.effort) * 40.0).astype(np.float32)
     assert np.array_equal(env.action_space.high, tau_max)                            # the action space of this mode
@@ -171,8 +61,8 @@ def test_torque_control_with_gravity():
 
 def test_config4_16384_envs_with_the_demo_obstacles():
     """BASELINE.json configs[3]: ground plane, the reference demo's box, a sphere; contact penalty in the reward."""
-    from pioneer_b200 import demo_obstacles
-    env, orc = make(16384, limit=50, obstacles=demo_obstacles(), penalty=0.5, seed=9, **PD)
+    env = dynamic_env(16384, obstacles=True, random_box=False, max_episode_steps=50, seed=9)
+    orc = c_dyn_oracle_for(env, 9)
     worst, n_done = lockstep(env, orc, 100, setpoints(env, 3), check_every=5)
     assert n_done >= 2 * 16384 and worst["free_fraction"] > 0.85
     print("config4 dynamic parity, worst:", worst)
@@ -180,13 +70,13 @@ def test_config4_16384_envs_with_the_demo_obstacles():
 
 
 def test_per_env_random_box_in_dynamic_mode():
-    from pioneer_b200 import demo_obstacles
     n = 4096
-    env, orc = make(n, limit=20, obstacles=demo_obstacles(), penalty=0.5, random_box=True, seed=21, **PD)
-    assert np.array_equal(env.boxes().cpu().numpy().astype(np.float64), orc.state()["box"])
+    env = dynamic_env(n, obstacles=True, max_episode_steps=20, seed=21)
+    orc = c_dyn_oracle_for(env, 21)
+    assert np.array_equal(host_boxes(env), orc.state()["box"])
     worst, n_done = lockstep(env, orc, 45, setpoints(env, 5), check_every=5)
     assert n_done >= 2 * n
-    assert np.array_equal(env.boxes().cpu().numpy().astype(np.float64), orc.state()["box"])   # redrawn twice, same draws
+    assert np.array_equal(host_boxes(env), orc.state()["box"])      # redrawn twice, same draws
     env.close()
 
 
@@ -196,10 +86,10 @@ def test_bullet_like_stepping_against_the_compiled_oracle():
     (oracle/dynamics_oracle.c, stepping = 1), 4,096 envs x 60 steps with gravity, TimeLimit 25 and auto-reset.  The motor solve
     divides by dt, so qd carries 240 x the float32 rounding of q: bars |dq| <= 5e-5 + 5e-6 |q|, |dqd| <= 2e-3 + 2e-4 |qd|."""
     n = 4096
-    bullet = dict(link_damping=0.04, max_velocity=100.0, motor_kp=0.1, motor_kd=1.0, motor_max_force=5e4)
-    env, orc = make(n, limit=25, seed=14, gravity=9.81, bullet=bullet)
+    env = dynamic_env(n, control="bullet", max_episode_steps=25, seed=14)
+    orc = c_dyn_oracle_for(env, 14)
     assert np.array_equal(env.action_space.low, env.r_lo)                  # motor set points
-    worst, n_done = lockstep(env, orc, 60, setpoints(env, 9, hold=12), check_every=4, bars=(5e-5, 5e-6, 2e-3, 2e-4))
+    worst, n_done = lockstep(env, orc, 60, setpoints(env, 9, hold=12), check_every=4, bars=BULLET_BARS)
     assert n_done >= 2 * n and worst["free_fraction"] > 0.5
     print("bullet-like stepping, worst:", worst)
     env.close()
@@ -212,7 +102,8 @@ def test_free_running_drift_is_bounded_under_pd_control():
     the two differ by up to qd * dt -- 26 rad/s x 1/240 s = 0.11 rad -- until the controller pulls them together again); flags may only differ where the
     distance sits within that drift of the done threshold (never, for random targets)."""
     n = 8192
-    env, orc = make(n, limit=100, seed=31, **PD)
+    env = dynamic_env(n, max_episode_steps=100, seed=31)
+    orc = c_dyn_oracle_for(env, 31)
     fn = setpoints(env, 7, hold=50)
     worst, worst_q999 = 0.0, 0.0
     for t in range(300):

@@ -9,9 +9,9 @@ torch = pytest.importorskip("torch")
 
 from oracle.reach_oracle import OracleChain, OracleConfig, OracleEnv, contact_depth
 from pioneer_b200 import demo_obstacles
+from tests._gpu import PENALTY, c_oracle_for, host_boxes, kinematic_env
 
 pytestmark = pytest.mark.gpu
-PENALTY = 0.5
 
 
 def make(n, obstacles, penalty=PENALTY, mode="kinematic", **kw):
@@ -114,16 +114,11 @@ def test_config4_16384_envs_against_the_compiled_oracle(random_box):
     """BASELINE.json configs[3] in the kinematic mode: 16,384 envs x 60 steps with TimeLimit 25 (two auto-resets, which
     redraw the per-env box when random_box is on) against oracle/reach_oracle.c: joint state and flags bit-exact, reward
     (which carries the contact penalty) within 2e-3."""
-    from oracle.c_oracle import COracleBatch
-    from pioneer_b200 import BatchConfig, BatchedPioneerEnv
-    n, obstacles = 16384, demo_obstacles()
-    bc = BatchConfig(obstacles=obstacles, contact_penalty=PENALTY, max_episode_steps=25, auto_reset=True, random_box=random_box)
-    env = BatchedPioneerEnv(n, batch_config=bc, seed=77)
-    cfg = OracleConfig(obstacles=oracle_obstacles(obstacles), contact_penalty=PENALTY, max_episode_steps=25,
-                       random_box=(bc.box_pos_lo, bc.box_pos_hi, bc.box_size_lo, bc.box_size_hi) if random_box else None)
-    orc = COracleBatch(OracleChain.from_model(env.chain), n, cfg, seed=77)
+    n = 16384
+    env = kinematic_env(n, obstacles=True, random_box=random_box, max_episode_steps=25, auto_reset=True, seed=77)
+    orc = c_oracle_for(env, 77)
     if random_box:
-        assert np.array_equal(env.boxes().cpu().numpy().astype(np.float64), orc.boxes())
+        assert np.array_equal(host_boxes(env), orc.boxes())
     rng = np.random.default_rng(3)
     worst = 0.0
     for t in range(60):
@@ -136,13 +131,14 @@ def test_config4_16384_envs_against_the_compiled_oracle(random_box):
     assert np.array_equal(s["r"].cpu().numpy(), o["r"]) and np.array_equal(s["v"].cpu().numpy(), o["v"])
     assert worst <= 2e-3, worst
     if random_box:
-        assert np.array_equal(env.boxes().cpu().numpy().astype(np.float64), orc.boxes())
+        assert np.array_equal(host_boxes(env), orc.boxes())
     st = env.episode_stats()
     assert st["episodes"] == orc.stats[0] == 2 * n
     env.close()
 
 
 def test_oracle_env_applies_the_penalty():
+    """The CPU oracle on its own, so both of its configurations are written by hand."""
     from pioneer_b200.urdf import flatten_urdf
     chain = OracleChain.from_model(flatten_urdf())
     obstacles = oracle_obstacles(demo_obstacles())

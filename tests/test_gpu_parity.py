@@ -15,47 +15,18 @@ import pytest
 
 torch = pytest.importorskip("torch")
 
-from oracle.reach_oracle import PNR_DONE, PNR_TRUNCATED, OracleBatch, OracleConfig
-from tests._util import golden_case, load_golden, oracle_chain
+from oracle.reach_oracle import PNR_DONE, PNR_TRUNCATED
+from tests._gpu import POS_COLS, POS_TOL, REW_TOL, TRIG_COLS, TRIG_TOL, VALUE_COLS, c_oracle_for, check_obs, kinematic_env
+from tests._util import golden_case, load_golden
 
 pytestmark = pytest.mark.gpu
-
-POS_TOL = 2e-4
-REW_TOL = 1e-3
-TRIG_TOL = 5e-7
-
-# observation columns (pioneer_knm_env.py:194-211): value blocks and their cos / sin blocks
-VALUE_COLS = np.r_[0:6, 18:24, 36:42, 54:60, 72:78, 90:96, 108:114, 129:132]
-TRIG_COLS = np.r_[6:18, 24:36, 42:54, 60:72, 78:90, 96:108, 114:126]
-POS_COLS = np.r_[126:129, 132:136]
-
-
-def make_env(n, **kw):
-    from pioneer_b200 import BatchConfig, BatchedPioneerEnv, PioneerKinematicConfig
-    bc_keys = ("max_episode_steps", "auto_reset", "obs_mode", "arith")
-    bc = BatchConfig(**{k: kw.pop(k) for k in bc_keys if k in kw})
-    pc = kw.pop("pioneer_config", None)
-    if isinstance(pc, dict):
-        pc = PioneerKinematicConfig(**pc)
-    return BatchedPioneerEnv(n, batch_config=bc, pioneer_config=pc, **kw)
-
-
-def check_obs(obs_gpu, obs_ref, what=""):
-    obs_gpu = np.asarray(obs_gpu, np.float64)
-    obs_ref = np.asarray(obs_ref, np.float64)
-    assert np.array_equal(obs_gpu[..., VALUE_COLS], obs_ref[..., VALUE_COLS].astype(np.float32)), what
-    np.testing.assert_allclose(obs_gpu[..., TRIG_COLS], obs_ref[..., TRIG_COLS], rtol=0, atol=TRIG_TOL, err_msg=what)
-    np.testing.assert_allclose(obs_gpu[..., POS_COLS], obs_ref[..., POS_COLS], rtol=0, atol=POS_TOL, err_msg=what)
-    np.testing.assert_allclose(obs_gpu[..., 136], obs_ref[..., 136], rtol=0, atol=REW_TOL, err_msg=what)
-
-
 G = load_golden()
 
 
 def replay_golden(name, pioneer_config=None):
     """One env driven exactly like tests/golden/make_golden.py::rollout drove the reference."""
     case = golden_case(G, name)
-    env = make_env(1, max_episode_steps=500, auto_reset=False, pioneer_config=pioneer_config)
+    env = kinematic_env(1, max_episode_steps=500, auto_reset=False, **(pioneer_config or {}))
     ep = 0
     first = env.reset_world(case["q0"][ep][None], case["target"][ep][None], observe=True).cpu().numpy()[0]
     check_obs(first, case["reset_obs"][ep], f"{name} reset obs")
@@ -95,7 +66,7 @@ def test_golden_reward_knobs():
 
 def test_golden_multi_env_batch():
     """16 envs x 200 steps in ONE batch (a half-filled warp tile); env 0 is the cfg1 trajectory."""
-    env = make_env(16, max_episode_steps=500, auto_reset=False)
+    env = kinematic_env(16, max_episode_steps=500, auto_reset=False)
     env.reset_world(G["multi__q0"], G["multi__target"])
     actions = torch.as_tensor(G["multi__actions"]).cuda()
     for t in range(200):
@@ -115,12 +86,9 @@ def test_golden_multi_env_batch():
 # ---------------------------------------------------------------------------------------------
 def run_vs_oracle(n, steps, arith, obs_mode, max_episode_steps, seed, env_id_base=0, action_scale=1.0,
                   near_targets=False):
-    chain = oracle_chain()
-    cfg = OracleConfig(max_episode_steps=max_episode_steps)
-    ob = OracleBatch(chain, n, cfg, arith={"f32": "np2", "legacy64": "legacy"}[arith], env_id_base=env_id_base,
-                     seed=seed, auto_reset=True, obs_mode=obs_mode)
-    env = make_env(n, max_episode_steps=max_episode_steps, auto_reset=True, obs_mode=obs_mode, arith=arith,
-                   seed=seed, env_id_base=env_id_base)
+    env = kinematic_env(n, max_episode_steps=max_episode_steps, auto_reset=True, obs_mode=obs_mode, arith=arith,
+                        seed=seed, env_id_base=env_id_base)
+    ob = c_oracle_for(env, seed, compiled=False)
     # both sides were created reset with tick 0: same Philox draws
     s = env.state()
     os_ = ob.state()
@@ -192,7 +160,7 @@ def test_single_env_and_tiny_batches():
 # ---------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("n", [4096, 65536])
 def test_invariants_full_size(n):
-    env = make_env(n, max_episode_steps=500, auto_reset=True, seed=3)
+    env = kinematic_env(n, max_episode_steps=500, auto_reset=True, seed=3)
     obs0 = env.reset()
     # (i) after reset: a = v = 0, potential = 0 -> obs[90:126] = {0,1,0,0,1,0} pattern, obs[136] = 0
     o = obs0.cpu().numpy()
@@ -242,7 +210,7 @@ def test_invariants_full_size(n):
 def test_time_limit_and_zero_action_properties():
     """(iii) a == 0 forever: r constant, reward == -0.01 from step 2 on; (vii) done at step 500 whatever the distance."""
     n = 4096
-    env = make_env(n, max_episode_steps=500, auto_reset=True, seed=11)
+    env = kinematic_env(n, max_episode_steps=500, auto_reset=True, seed=11)
     obs0 = env.reset().clone()
     zero = torch.zeros((n, 6), device="cuda")
     for t in range(1, 501):
@@ -264,9 +232,9 @@ def test_time_limit_and_zero_action_properties():
 def test_sharding_is_invisible():
     """Two handles covering global ids [0, 3000) and [3000, 6000) reproduce one handle of 6000 envs bit for bit."""
     n = 6000
-    whole = make_env(n, max_episode_steps=5, seed=21)
-    lo = make_env(3000, max_episode_steps=5, seed=21, env_id_base=0)
-    hi = make_env(3000, max_episode_steps=5, seed=21, env_id_base=3000)
+    whole = kinematic_env(n, max_episode_steps=5, seed=21)
+    lo = kinematic_env(3000, max_episode_steps=5, seed=21, env_id_base=0)
+    hi = kinematic_env(3000, max_episode_steps=5, seed=21, env_id_base=3000)
     g = torch.Generator(device="cuda").manual_seed(1)
     a_max = torch.as_tensor(whole.a_max).cuda()
     for t in range(12):
@@ -284,8 +252,8 @@ def test_sharding_is_invisible():
 
 def test_step_host_matches_step_tensor():
     n = 1000
-    a_env = make_env(n, max_episode_steps=6, seed=5)
-    b_env = make_env(n, max_episode_steps=6, seed=5)
+    a_env = kinematic_env(n, max_episode_steps=6, seed=5)
+    b_env = kinematic_env(n, max_episode_steps=6, seed=5)
     rng = np.random.default_rng(0)
     for t in range(8):
         act = (rng.uniform(-1, 1, size=(n, 6)) * a_env.a_max).astype(np.float32)
@@ -298,7 +266,7 @@ def test_step_host_matches_step_tensor():
 
 def test_reset_subset_and_observe_indices():
     n = 100
-    env = make_env(n, max_episode_steps=0, auto_reset=False, seed=2)
+    env = kinematic_env(n, max_episode_steps=0, auto_reset=False, seed=2)
     before = env.state()
     idx = [3, 50, 99]
     q0 = np.zeros((3, 6), np.float32)
@@ -325,7 +293,7 @@ def test_fk_known_answers_on_device():
         (0, 0, 0, 0, 0, 0.5): (14.6, 0.089091476652, 15.667406867592),
         (0.3, -0.4, 0.9, 1.1, -0.7, 2.0): (7.904033967723, 1.072102752440, 5.624962379045),
     }
-    env = make_env(len(kat), max_episode_steps=0, auto_reset=False)
+    env = kinematic_env(len(kat), max_episode_steps=0, auto_reset=False)
     q = np.array(list(kat.keys()), np.float32)
     obs = env.reset_world(q, np.zeros((len(kat), 3), np.float32), observe=True).cpu().numpy()
     np.testing.assert_allclose(obs[:, 126:129], np.array(list(kat.values())), atol=2e-5)
@@ -334,7 +302,7 @@ def test_fk_known_answers_on_device():
 
 def test_errors_are_loud():
     from pioneer_b200 import _cabi
-    env = make_env(8)
+    env = kinematic_env(8)
     with pytest.raises(_cabi.PioneerB200Error):
         _cabi.check(env._lib.pnr_step(env._h, None, None, None, None, None), "pnr_step")
     with pytest.raises(_cabi.PioneerB200Error):
@@ -347,11 +315,9 @@ def test_errors_are_loud():
 # restatement, oracle/reach_oracle.c): per-step q / qdot / pointer diff, done/reset masks bit-exact.
 # ---------------------------------------------------------------------------------------------
 def test_cfg2_4096_envs_1000_steps_vs_c_oracle():
-    from oracle.c_oracle import COracleBatch
     n, steps, seed = 4096, 1000, 2026
-    chain = oracle_chain()
-    cc = COracleBatch(chain, n, OracleConfig(max_episode_steps=500), arith="np2", seed=seed, obs_mode="terminal")
-    env = make_env(n, max_episode_steps=500, auto_reset=True, obs_mode="terminal", seed=seed)
+    env = kinematic_env(n, max_episode_steps=500, auto_reset=True, obs_mode="terminal", seed=seed)
+    cc = c_oracle_for(env, seed)
     rng = np.random.default_rng(7)
     worst = dict(pos=0.0, rew=0.0, trig=0.0)
     n_done = 0
@@ -385,11 +351,10 @@ def test_deep_grid_stride_pipeline_vs_c_oracle(n):
     """Many tiles per CTA (the producer / consumer pipeline over two tile buffers runs 10-55 iterations deep):
     every row against the C oracle, plus run-to-run bit-identity of two handles (a barrier protocol error or a
     tile-buffer race would show up as a mismatch somewhere in 10^6 rows)."""
-    from oracle.c_oracle import COracleBatch
     seed, steps = 77, 3
-    cc = COracleBatch(oracle_chain(), n, OracleConfig(max_episode_steps=2), arith="np2", seed=seed, obs_mode="terminal")
-    a = make_env(n, max_episode_steps=2, auto_reset=True, obs_mode="terminal", seed=seed)
-    b = make_env(n, max_episode_steps=2, auto_reset=True, obs_mode="terminal", seed=seed)
+    a = kinematic_env(n, max_episode_steps=2, auto_reset=True, obs_mode="terminal", seed=seed)
+    b = kinematic_env(n, max_episode_steps=2, auto_reset=True, obs_mode="terminal", seed=seed)
+    cc = c_oracle_for(a, seed)
     g = torch.Generator(device="cuda").manual_seed(5)
     a_max = torch.as_tensor(a.a_max).cuda()
     for t in range(steps):
@@ -415,9 +380,8 @@ def test_non_finite_and_degenerate_actions_follow_the_reference_arithmetic():
     NaN propagates through every comparison, +-inf saturates the velocity with a zero first phase, a = -eps makes the
     divisor of the saturation time exactly zero.  Same bits as the oracle, NaN for NaN."""
     n = 64
-    chain = oracle_chain()
-    ob = OracleBatch(chain, n, OracleConfig(max_episode_steps=0), arith="np2", seed=8, auto_reset=False)
-    env = make_env(n, max_episode_steps=0, auto_reset=False, seed=8)
+    env = kinematic_env(n, max_episode_steps=0, auto_reset=False, seed=8)
+    ob = c_oracle_for(env, 8, compiled=False)
     rng = np.random.default_rng(0)
     eps32 = np.float32(1e-5)
     specials = np.array([np.nan, np.inf, -np.inf, 3e38, -3e38, -eps32, 0.0, -0.0, 1e-40, 1.2e5, -1.2e5], np.float32)
@@ -461,7 +425,6 @@ def test_randomised_configs_vs_c_oracle(case):
     """Every knob of PioneerKinematicConfig / SimulationConfig / TimeLimit travels through pnr_config into the kernel:
     randomised settings (limits ratios, done distance, reward shaping, target box, timestep, frame_skip) against the C
     oracle on the same seeds and actions."""
-    from oracle.c_oracle import COracleBatch
     from pioneer_b200 import BatchConfig, BatchedPioneerEnv, PioneerKinematicConfig, SimulationConfig
     rng = np.random.default_rng(1000 + case)
     lo = rng.uniform([-5, -12, 0], [10, -2, 3])
@@ -472,11 +435,10 @@ def test_randomised_configs_vs_c_oracle(case):
               penalty_step=float(rng.uniform(0, 0.1)), target_lo=tuple(lo), target_hi=tuple(hi))
     timestep, frame_skip, limit = float(rng.uniform(1 / 480, 1 / 60)), int(rng.integers(1, 20)), int(rng.integers(3, 12))
     n, seed = 2048 + case, 40 + case
-    cc = COracleBatch(oracle_chain(), n, OracleConfig(max_episode_steps=limit, timestep=timestep, frame_skip=frame_skip, **kw),
-                      arith="np2", seed=seed, env_id_base=5 * case)
     env = BatchedPioneerEnv(n, seed=seed, env_id_base=5 * case, pioneer_config=PioneerKinematicConfig(**kw),
                             simulation_config=SimulationConfig(timestep=timestep, frame_skip=frame_skip),
                             batch_config=BatchConfig(max_episode_steps=limit))
+    cc = c_oracle_for(env, seed)
     assert np.array_equal(env.a_max, cc.a_max) and np.array_equal(env.v_max, cc.v_max)
     reached = 0
     for t in range(30):

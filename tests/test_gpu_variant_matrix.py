@@ -18,51 +18,12 @@ import pytest
 
 torch = pytest.importorskip("torch")
 
-from oracle.c_oracle import COracleBatch
 from oracle.filter_oracle import BatchSyncFilter
-from oracle.reach_oracle import OracleChain, OracleConfig
-from tests.test_gpu_dynamic_parity import PD, lockstep, make as make_dyn_with_oracle, setpoints
-from tests.test_gpu_parity import check_obs
+from tests._gpu import (BULLET_BARS, c_dyn_oracle_for, c_oracle_for, check_obs, dynamic_env, fragment_buffers,
+                        fragments_equal_single_steps, host_boxes, k1_fragments_vs_c_oracle, kinematic_env, lockstep,
+                        setpoints, uniform_actions)
 
 pytestmark = pytest.mark.gpu
-
-PENALTY = 0.5
-BULLET = dict(link_damping=0.04, max_velocity=100.0, motor_kp=0.1, motor_kd=1.0, motor_max_force=5e4)
-BULLET_BARS = (5e-5, 5e-6, 2e-3, 2e-4)          # test_gpu_dynamic_parity.py: the motor solve divides by dt
-STATE_KEYS = ("r", "v", "a", "potential", "target", "t", "ep_return")
-
-
-def kin_env(n, arith="f32", obs_mode="terminal", limit=7, obstacles=False, seed=0):
-    """Kinematic env; obstacles=True: the demo obstacles, contact penalty 0.5 and a box redrawn at every reset."""
-    from pioneer_b200 import BatchConfig, BatchedPioneerEnv, demo_obstacles
-    bc = BatchConfig(max_episode_steps=limit, auto_reset=True, obs_mode=obs_mode, arith=arith,
-                     obstacles=demo_obstacles() if obstacles else [], contact_penalty=PENALTY if obstacles else 0.0,
-                     random_box=obstacles)
-    return BatchedPioneerEnv(n, batch_config=bc, seed=seed)
-
-
-def kin_oracle(env, seed):
-    bc = env.batch_config
-    cfg = OracleConfig(max_episode_steps=bc.max_episode_steps, contact_penalty=bc.contact_penalty,
-                       obstacles=tuple((o.kind, o.position, o.extent) for o in bc.obstacles),
-                       random_box=(bc.box_pos_lo, bc.box_pos_hi, bc.box_size_lo, bc.box_size_hi) if bc.random_box else None)
-    return COracleBatch(OracleChain.from_model(env.chain), env.n_envs, cfg, arith={"f32": "np2", "legacy64": "legacy"}[bc.arith],
-                        seed=seed, obs_mode=bc.obs_mode)
-
-
-def dyn_env(n, obs_mode="terminal", limit=5, obstacles=False, stepping="explicit", seed=0):
-    """Dynamic env: PD control (bench.py's workload) or Bullet-like motors under gravity, as test_gpu_dynamic_parity.py."""
-    from pioneer_b200 import BatchConfig, BatchedPioneerEnv, SimulationConfig, demo_obstacles
-    ctrl = dict(kp=PD["kp"], kd=PD["kd"], torque_scale=PD["torque_scale"]) if stepping == "explicit" \
-        else dict(stepping="bullet", **BULLET)
-    bc = BatchConfig(mode="dynamic", max_episode_steps=limit, auto_reset=True, obs_mode=obs_mode,
-                     obstacles=demo_obstacles() if obstacles else [], contact_penalty=PENALTY if obstacles else 0.0,
-                     random_box=obstacles, **ctrl)
-    return BatchedPioneerEnv(n, batch_config=bc, simulation_config=SimulationConfig(gravity=9.81), seed=seed)
-
-
-def host_boxes(env):
-    return env.boxes().cpu().numpy().astype(np.float64)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -74,8 +35,8 @@ def test_kinematic_obstacles_single_step_vs_c_oracle(arith, obs_mode, n):
     """TimeLimit 7 over 24 steps: three auto-resets per env, each redrawing the env's box; 77 envs = two full warp tiles and
     a ragged one.  In auto-reset observation mode a finished row shows the oracle's fresh episode."""
     seed, steps = 31, 24
-    env = kin_env(n, arith, obs_mode, limit=7, obstacles=True, seed=seed)
-    orc = kin_oracle(env, seed)
+    env = kinematic_env(n, arith=arith, obs_mode=obs_mode, max_episode_steps=7, obstacles=True, seed=seed)
+    orc = c_oracle_for(env, seed)
     assert np.array_equal(host_boxes(env), orc.boxes())
     rng = np.random.default_rng(seed)
     worst_rew, n_done = 0.0, 0
@@ -113,63 +74,14 @@ def test_kinematic_obstacles_single_step_vs_c_oracle(arith, obs_mode, n):
 # ---------------------------------------------------------------------------------------------
 # 2. fragments (pnr_step_many) equal single steps (pnr_step), bit for bit, for every combination
 # ---------------------------------------------------------------------------------------------
-def fragments_equal_single_steps(make, fused, T=8, fragments=3, seed=0):
-    """Twin envs: `a` runs fragments of T steps in one launch, `b` the same actions one step per launch.  With the fused
-    filter a first fragment is compared under the identity (nothing synchronised yet), then both sides synchronise and are
-    given the same statistics, so that the compared fragments normalise with non-trivial applied statistics."""
+def twins_equal(make, fused, seed):
+    """Fragments of 8 against single steps on twin envs (three fragments, after a first one under the identity filter
+    when the fused filter is on)."""
     from pioneer_b200.obs_filter import MeanStdObsFilter
     a, b = make(), make()
-    n = a.n_envs
-    fa, fb = (MeanStdObsFilter(a, fused=True), MeanStdObsFilter(b, fused=True)) if fused else (None, None)
-    g = torch.Generator(device="cuda").manual_seed(seed)
-    lo, hi = torch.as_tensor(a.action_space.low).cuda(), torch.as_tensor(a.action_space.high).cuda()
-    n_pad = (n + 3) // 4 * 4                      # every obs[t] on a 16-byte boundary
-    obs = torch.empty((T, n_pad, 137), device="cuda")[:, :n]
-    rew = torch.empty((T, n), device="cuda")
-    flg = torch.empty((T, n), dtype=torch.uint8, device="cuda")
-    n_done = 0
-
-    def fragment(k):
-        nonlocal n_done
-        act = lo + torch.rand((T, n, 6), device="cuda", generator=g) * (hi - lo)
-        a.step_many(act, obs, rew, flg)
-        for t in range(T):
-            o, r, f = b.step_tensor(act[t])
-            assert torch.equal(f, flg[t]), (k, t, int((f != flg[t]).sum()))
-            assert torch.equal(r, rew[t]), (k, t, float((r - rew[t]).abs().max()))
-            assert torch.equal(o, obs[t]), (k, t, float((o - obs[t]).abs().max()))
-        sa, sb = a.state(), b.state()
-        for key in STATE_KEYS:
-            assert torch.equal(sa[key], sb[key]), (k, key)
-        if a.batch_config.random_box:              # only a random-box handle keeps per-env boxes
-            assert torch.equal(a.boxes(), b.boxes()), k
-        n_done += int((flg & 1).sum())
-
-    def same_filter_statistics():
-        fa.sync(); fb.sync()
-        (na, ma, va), (nb, mb, vb) = fa._get(), fb._get()
-        assert na == nb                            # float64 atomics in a different order: sums agree to rounding
-        np.testing.assert_allclose(ma, mb, rtol=1e-9, atol=1e-12)
-        np.testing.assert_allclose(va, vb, rtol=1e-9, atol=1e-12)
-        return na, ma, va
-
-    if fused:
-        fragment(-1)
-        stats = same_filter_statistics()
-        assert np.abs(stats[1]).max() > 1.0        # the applied statistics are no longer the identity
-        fa.set_stats(*stats); fb.set_stats(*stats)
-    for k in range(fragments):
-        fragment(k)
-    if fused:
-        same_filter_statistics()
-    assert n_done > 0                              # resets (and box redraws) happened inside the fragments
-    st_a, st_b = a.episode_stats(), b.episode_stats()
-    for key in ("episodes", "sum_length", "env_steps", "reached_target", "max_return", "min_return"):
-        assert st_a[key] == st_b[key], (key, st_a[key], st_b[key])
-    # the return sums are float64 atomics, added per warp in an order that depends on the launch shape; the squared returns
-    # are rounded products, so their sum can differ in the last bits
-    for key in ("sum_return", "sum_return_sq"):
-        assert abs(st_a[key] - st_b[key]) <= 1e-9 * abs(st_b[key]), (key, st_a[key], st_b[key])
+    filters = (MeanStdObsFilter(a, fused=True), MeanStdObsFilter(b, fused=True)) if fused else None
+    fragments_equal_single_steps(a, b, T=8, fragments=3, generator=torch.Generator(device="cuda").manual_seed(seed),
+                                 filters=filters)
     a.close(); b.close()
 
 
@@ -185,7 +97,8 @@ KIN_CASES = [(arith, obs_mode, obstacles, False, SMALL) for arith in ("f32", "le
 def test_kinematic_fragment_equals_single_steps(arith, obs_mode, obstacles, fused, n):
     """K1 (the fused filter exists for float32 terminal observations only; the API refuses the rest).  TimeLimit 4 with
     fragments of 8: every env resets twice inside each fragment."""
-    fragments_equal_single_steps(lambda: kin_env(n, arith, obs_mode, limit=4, obstacles=obstacles, seed=6), fused, seed=1)
+    twins_equal(lambda: kinematic_env(n, arith=arith, obs_mode=obs_mode, max_episode_steps=4, obstacles=obstacles, seed=6),
+                fused, seed=1)
 
 
 DYN_CASES = [(obs_mode, obstacles, stepping, False, SMALL) for obs_mode in ("terminal", "autoreset")
@@ -199,8 +112,9 @@ DYN_CASES = [(obs_mode, obstacles, stepping, False, SMALL) for obs_mode in ("ter
 @pytest.mark.parametrize("obs_mode,obstacles,stepping,fused,n", DYN_CASES)
 def test_dynamic_fragment_equals_single_steps(obs_mode, obstacles, stepping, fused, n):
     """K2: the warp keeps its tile's env state in registers across the fragment; TimeLimit 5 with fragments of 8."""
-    fragments_equal_single_steps(lambda: dyn_env(n, obs_mode, limit=5, obstacles=obstacles, stepping=stepping, seed=8),
-                                 fused, seed=2)
+    control = "pd" if stepping == "explicit" else stepping
+    twins_equal(lambda: dynamic_env(n, control=control, obs_mode=obs_mode, max_episode_steps=5, obstacles=obstacles, seed=8),
+                fused, seed=2)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -210,31 +124,9 @@ def test_kinematic_obstacle_fragments_vs_c_oracle():
     """16,384 envs, random box, TimeLimit 25, eight fragments of 8 through pnr_step_many; the oracle steps eight times per
     fragment.  Flags and reward every step; r, v, boxes and the observation at the end of every fragment."""
     n, T, seed = 16384, 8, 44
-    env = kin_env(n, limit=25, obstacles=True, seed=seed)
-    orc = kin_oracle(env, seed)
-    rng = np.random.default_rng(seed)
-    obs = torch.empty((T, n, 137), device="cuda")
-    rew = torch.empty((T, n), device="cuda")
-    flg = torch.empty((T, n), dtype=torch.uint8, device="cuda")
-    worst, n_done = 0.0, 0
-    for k in range(8):
-        act = (rng.uniform(-1, 1, size=(T, n, 6)) * env.a_max).astype(np.float32)
-        env.step_many(torch.as_tensor(act).cuda(), obs, rew, flg)
-        rew_h, flg_h = rew.cpu().numpy(), flg.cpu().numpy()
-        for t in range(T):
-            o_obs, o_rew, o_flags = orc.step(act[t], want_obs=(t == T - 1))
-            assert np.array_equal(flg_h[t], o_flags), (k, t)
-            worst = max(worst, float(np.abs(rew_h[t] - o_rew).max()))
-            n_done += int((o_flags & 1).sum())
-        check_obs(obs[T - 1].cpu().numpy(), o_obs, f"fragment {k}")
-        s, o = env.state(), orc.state()
-        for key in ("r", "v", "a", "t"):
-            assert np.array_equal(s[key].cpu().numpy(), o[key]), (k, key)
-        assert np.array_equal(host_boxes(env), orc.boxes()), k
-    assert worst <= 2e-3, worst
+    env = kinematic_env(n, max_episode_steps=25, obstacles=True, seed=seed)
+    worst, n_done, _ = k1_fragments_vs_c_oracle(env, seed, T=T, fragments=8)
     assert n_done >= 2 * n
-    st = env.episode_stats()
-    assert st["episodes"] == orc.stats[0] == n_done and st["sum_length"] == orc.stats[2]
     print(f"K1 obstacle fragments vs C oracle, {n} envs x {8 * T} steps: worst reward deviation {worst:.3e}")
     env.close()
 
@@ -243,10 +135,9 @@ def test_kinematic_obstacle_fragments_vs_c_oracle():
 # 4. K2 lock step for the single-step instantiations test_gpu_dynamic_parity.py does not run
 # ---------------------------------------------------------------------------------------------
 def test_dynamic_obstacles_random_box_autoreset_lockstep():
-    from pioneer_b200 import demo_obstacles
     n = 4096
-    env, orc = make_dyn_with_oracle(n, obs_mode="autoreset", limit=20, obstacles=demo_obstacles(), penalty=PENALTY,
-                                    random_box=True, seed=23, **PD)
+    env = dynamic_env(n, obs_mode="autoreset", max_episode_steps=20, obstacles=True, seed=23)
+    orc = c_dyn_oracle_for(env, 23)
     assert np.array_equal(host_boxes(env), orc.state()["box"])
     worst, n_done = lockstep(env, orc, 45, setpoints(env, 11), obs_mode="autoreset", check_every=5)
     assert n_done >= 2 * n and worst["free_fraction"] > 0.85, (n_done, worst)
@@ -256,10 +147,9 @@ def test_dynamic_obstacles_random_box_autoreset_lockstep():
 
 
 def test_dynamic_bullet_stepping_with_obstacles_lockstep():
-    from pioneer_b200 import demo_obstacles
     n = 4096
-    env, orc = make_dyn_with_oracle(n, limit=25, obstacles=demo_obstacles(), penalty=PENALTY, random_box=True, seed=15,
-                                    gravity=9.81, bullet=BULLET)
+    env = dynamic_env(n, control="bullet", max_episode_steps=25, obstacles=True, seed=15)
+    orc = c_dyn_oracle_for(env, 15)
     assert np.array_equal(host_boxes(env), orc.state()["box"])
     worst, n_done = lockstep(env, orc, 60, setpoints(env, 12, hold=12), check_every=4, bars=BULLET_BARS)
     assert n_done >= 2 * n and worst["free_fraction"] > 0.5, (n_done, worst)
@@ -280,18 +170,15 @@ def test_fused_filter_statistics_at_scale_vs_float64(mode):
     per-lane partials) and after the second."""
     from pioneer_b200.obs_filter import MeanStdObsFilter
     n, T = (1 << 20, 8) if mode == "kinematic" else (131072, 8)
-    make = (lambda: kin_env(n, limit=6, seed=3)) if mode == "kinematic" else (lambda: dyn_env(n, limit=6, seed=3))
-    a, b = make(), make()
+    make = kinematic_env if mode == "kinematic" else dynamic_env
+    a, b = make(n, max_episode_steps=6, seed=3), make(n, max_episode_steps=6, seed=3)
     fa = MeanStdObsFilter(a, fused=True)
     g = torch.Generator(device="cuda").manual_seed(4)
-    lo, hi = torch.as_tensor(a.action_space.low).cuda(), torch.as_tensor(a.action_space.high).cuda()
-    obs_a, obs_b = (torch.empty((T, n, 137), device="cuda") for _ in range(2))
-    rew_a, rew_b = (torch.empty((T, n), device="cuda") for _ in range(2))
-    flg_a, flg_b = (torch.empty((T, n), dtype=torch.uint8, device="cuda") for _ in range(2))
+    (obs_a, rew_a, flg_a), (obs_b, rew_b, flg_b) = fragment_buffers(T, n), fragment_buffers(T, n)
     shift, s1, s2, rows = None, None, None, 0
     report = []
     for it in range(2):
-        act = lo + torch.rand((T, n, 6), device="cuda", generator=g) * (hi - lo)
+        act = uniform_actions(a, g, T)
         a.step_many(act, obs_a, rew_a, flg_a)
         b.step_many(act, obs_b, rew_b, flg_b)
         assert torch.equal(flg_a, flg_b) and torch.equal(rew_a, rew_b)
@@ -351,12 +238,9 @@ def test_rollout_worker_fused_filter_values_vs_the_filter_oracle(cuda_graph):
                 warm.append(w.actions.clone())
         w._steps = recording_steps
     ora = BatchSyncFilter(137)
-    n_pad = (n + 3) // 4 * 4                           # every step's rows on a 16-byte boundary
     act_buf = torch.empty((T, n, 6), device="cuda")
-    raw = torch.empty((T, n_pad, 137), device="cuda")[:, :n]
-    rows = torch.empty((T, n_pad, 137), device="cuda")[:, :n]
-    rew = torch.empty((T, n), device="cuda")
-    flg = torch.empty((T, n), dtype=torch.uint8, device="cuda")
+    raw, rew, flg = fragment_buffers(T, n)
+    rows = fragment_buffers(T, n)[0]
 
     def twin_steps(k):
         for t in range(k):
