@@ -3,7 +3,6 @@
 // registers, then the same task code as the kinematic env (pioneer_knm_env.py:151-211): forward kinematics of
 // the pointer, reward, done, TimeLimit, statistics, auto-reset, 137-float observation staged per warp in shared
 // memory and stored with one TMA bulk copy.  Bound: FP32 pipe (10 x ~1.45 kflop per env-step against 761 B).
-#include <cstdlib>
 #include "pnr_dynamic_kernel.cuh"
 
 cudaError_t pnr_launch_step_dynamic(const PnrParams& p, int device, int obs_mode, float4* state, const float* actions,
@@ -19,8 +18,7 @@ cudaError_t pnr_launch_step_dynamic(const PnrParams& p, int device, int obs_mode
     static int grids[PNR_MAX_DEVICES][2][3][2][2] = {};
     const int obst = p.n_obstacles > 0 ? 1 : 0;
     const int stepping = p.dyn_stepping == PNR_STEPPING_BULLET ? 1 : 0;
-    int chain = p.chain_kind == 1 ? (p.dyn_iso_links ? PNR_CHAIN_PIONEER_ISO : PNR_CHAIN_PIONEER) : PNR_CHAIN_GENERIC;
-    if (const char* e = getenv("PNR_DYN_CHAIN")) chain = atoi(e) < chain ? atoi(e) : chain;   // developer / test knob: force a less specialised kernel
+    const int chain = p.chain_kind == 1 ? (p.dyn_iso_links ? PNR_CHAIN_PIONEER_ISO : PNR_CHAIN_PIONEER) : PNR_CHAIN_GENERIC;
     Kern kern = stepping ? pnr_dynamic_bullet_kernel(chain, obs_mode, obst) : explicit_kernels[chain][obs_mode][obst];
     int& resident = grids[device % PNR_MAX_DEVICES][stepping][chain][obs_mode][obst];
     if (resident == 0) {

@@ -120,15 +120,19 @@ pnr_filter_kernel(const float* __restrict__ in, float* __restrict__ out, int64_t
     if (update && blockIdx.x == 0 && tid == 0) atomicAdd(&delta[0], (double)n_rows);
 }
 
-// copy 0 += copies 1 .. SLOTS-1, which are cleared (see pnr_launch.h)
+// column j of the accumulator summed over its copies (see pnr_launch.h) in copy order, as every reader folds it
+__device__ __forceinline__ double pnr_filter_fold_column(const double* slots, int j) {
+    double acc = slots[j];
+    for (int s = 1; s < PNR_FILTER_SLOTS; ++s) acc += slots[(size_t)s * PNR_FILTER_DELTA_LEN + j];
+    return acc;
+}
+
+// copy 0 += copies 1 .. SLOTS-1, which are cleared
 __global__ void pnr_filter_fold_kernel(double* __restrict__ slots) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= PNR_FILTER_DELTA_LEN) return;
-    double acc = slots[c];
-    for (int s = 1; s < PNR_FILTER_SLOTS; ++s) {
-        acc += slots[(size_t)s * PNR_FILTER_DELTA_LEN + c];
-        slots[(size_t)s * PNR_FILTER_DELTA_LEN + c] = 0.0;
-    }
+    const double acc = pnr_filter_fold_column(slots, c);
+    for (int s = 1; s < PNR_FILTER_SLOTS; ++s) slots[(size_t)s * PNR_FILTER_DELTA_LEN + c] = 0.0;
     slots[c] = acc;
 }
 
@@ -151,9 +155,6 @@ __global__ void pnr_filter_refresh_kernel(const double* state, float* applied, i
     if (c < PNR_OBS_DIM) pnr_filter_refresh_column(state[0], state[1 + c], state[1 + PNR_OBS_DIM + c], applied, c, demean, destd);
 }
 
-// Once per iteration, entirely on the device (one CTA, thread = column): fold the accumulator copies (or take `merged`,
-// the all-reduced delta of all ranks), merge into the running count / mean / M2 (Chan et al.; the batch sums are relative
-// to the APPLIED mean, i.e. what the kernels subtracted), refresh the applied statistics, clear the accumulator.
 // Chan et al. merge of one column's batch sums (relative to the APPLIED mean) into the running mean / M2, and the refreshed
 // applied statistics of that column; na = running count before, nb = rows in the batch, n = count after
 __device__ __forceinline__ void pnr_filter_merge_column(int c, double na, double nb, double n, double sum_d, double sum_q,
@@ -180,29 +181,29 @@ __device__ __forceinline__ void pnr_filter_clear_slots(double* slots, int c, boo
     }
 }
 
-__global__ void __launch_bounds__(PNR_FILTER_THREADS)
-pnr_filter_sync_kernel(double* slots, const double* merged, double* state, float* applied, int demean, int destd) {
-    // no __restrict__ here: the count is written by one thread and every thread carries its own copy of the new value
+// One CTA, thread = column: merge a batch (nb rows; this column's sums, relative to the applied mean) into the running
+// count / mean / M2, refresh the applied statistics, clear the accumulator.  No __restrict__: one thread writes the count.
+__device__ __forceinline__ void pnr_filter_merge_batch(double nb, double sum_d, double sum_q, double* slots, double* state,
+                                                       float* applied, int demean, int destd) {
     const int c = threadIdx.x;
     const bool col_ok = c < PNR_OBS_DIM;
-    double nb, sum_d = 0.0, sum_q = 0.0;
-    if (merged) {
-        nb = merged[0];
-        if (col_ok) { sum_d = merged[1 + c]; sum_q = merged[1 + PNR_OBS_DIM + c]; }
-    } else {
-        nb = 0.0;
-        for (int k = 0; k < PNR_FILTER_SLOTS; ++k) {
-            const double* sl = slots + (size_t)k * PNR_FILTER_DELTA_LEN;
-            nb += sl[0];
-            if (col_ok) { sum_d += sl[1 + c]; sum_q += sl[1 + PNR_OBS_DIM + c]; }
-        }
-    }
     const double na = state[0];
     const double n = nb > 0.0 ? na + nb : na;
     __syncthreads();                                            // everybody has read the old count and the accumulator
     if (col_ok) pnr_filter_merge_column(c, na, nb, n, sum_d, sum_q, state, applied, demean, destd);
     if (c == 0) state[0] = n;
-    pnr_filter_clear_slots(slots, c, col_ok);                   // clear the accumulator
+    pnr_filter_clear_slots(slots, c, col_ok);
+}
+
+// Once per iteration, entirely on the device: the batch is `merged` (the merged delta of all ranks) or else this rank's
+// accumulator, folded
+__global__ void __launch_bounds__(PNR_FILTER_THREADS)
+pnr_filter_sync_kernel(double* slots, const double* merged, double* state, float* applied, int demean, int destd) {
+    const int c = threadIdx.x;
+    const bool col_ok = c < PNR_OBS_DIM;
+    auto batch = [&](int j) { return merged ? merged[j] : pnr_filter_fold_column(slots, j); };
+    pnr_filter_merge_batch(batch(0), col_ok ? batch(1 + c) : 0.0, col_ok ? batch(1 + PNR_OBS_DIM + c) : 0.0, slots, state,
+                           applied, demean, destd);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -253,8 +254,7 @@ pnr_iteration_sync_kernel(PnrStats* stats, int clear, double* filt_slots, double
     if (i < PNR_STATS_LEN) {
         v = pnr_stats_read(stats, i);
     } else if (i < len) {
-        const int j = i - PNR_STATS_LEN;
-        for (int k = 0; k < PNR_FILTER_SLOTS; ++k) v += filt_slots[(size_t)k * PNR_FILTER_DELTA_LEN + j];
+        v = pnr_filter_fold_column(filt_slots, i - PNR_STATS_LEN);
     }
     __syncthreads();                                            // every field is read before the window is cleared
     if (i == 0 && clear) pnr_stats_clear(stats);
@@ -299,18 +299,13 @@ pnr_iteration_sync_kernel(PnrStats* stats, int clear, double* filt_slots, double
     if (!filt_slots) return;
     merged_s[i] = acc;
     __syncthreads();
-    const int c = i;
-    const bool col_ok = c < PNR_OBS_DIM;
-    const double nb = merged_s[PNR_STATS_LEN];
-    const double na = filt_state[0];
-    const bool usable = nb == nb;                               // a poisoned (timed-out) exchange leaves the filter alone
-    const double n = (usable && nb > 0.0) ? na + nb : na;
-    __syncthreads();                                            // everybody has read the old count
-    if (col_ok && usable)
-        pnr_filter_merge_column(c, na, nb, n, merged_s[PNR_STATS_LEN + 1 + c], merged_s[PNR_STATS_LEN + 1 + PNR_OBS_DIM + c],
-                                filt_state, applied, demean, destd);
-    if (c == 0) filt_state[0] = n;
-    pnr_filter_clear_slots(filt_slots, c, col_ok);
+    const double* batch = merged_s + PNR_STATS_LEN;             // [count, sum_d[137], sum_q[137]]
+    const bool col_ok = i < PNR_OBS_DIM;
+    if (batch[0] == batch[0])
+        pnr_filter_merge_batch(batch[0], col_ok ? batch[1 + i] : 0.0, col_ok ? batch[1 + PNR_OBS_DIM + i] : 0.0, filt_slots,
+                               filt_state, applied, demean, destd);
+    else                    // a poisoned (timed-out) exchange leaves the statistics alone; the accumulator is still cleared
+        pnr_filter_clear_slots(filt_slots, i, col_ok);
 }
 
 cudaError_t pnr_launch_filter_refresh(const double* state, float* applied, int demean, int destd, cudaStream_t stream) {

@@ -13,6 +13,7 @@ from typing import Dict, Optional, Tuple
 import torch
 import torch.distributed as dist
 
+from . import _cabi
 from .batched_env import STATS_FIELDS
 
 
@@ -51,19 +52,23 @@ def shard_range(total_envs: int, rank: int, world_size: int) -> Tuple[int, int]:
     return base, n_local
 
 
-def _merge(gathered: torch.Tensor) -> torch.Tensor:
-    """[world, len] -> [len]: SUM over the counters and extras, MAX / MIN over slots 4 / 5.  On a GPU this is ONE kernel of
-    the library (pnr_stats_merge_device) on the current stream; on the CPU (gloo tests) plain torch."""
+def _gather_merge(packed: torch.Tensor, gathered: torch.Tensor, out: torch.Tensor,
+                  group: Optional[dist.ProcessGroup] = None, stream: Optional[int] = None) -> torch.Tensor:
+    """Every rank's ``packed`` vector all-gathered into ``gathered`` [world, len] (one NCCL all-gather on the GPU, gloo on
+    the CPU; none at world 1, where ``gathered`` is ``packed`` itself) and merged into ``out`` [len]: SUM over the counters
+    and extras, MAX / MIN over slots 4 / 5.  On a GPU the merge is ONE kernel of the library (pnr_stats_merge_device) on
+    ``stream``, which belongs to the current device; on the CPU plain torch."""
     world, k = gathered.shape
+    if world > 1:
+        if packed.is_cuda:
+            dist.all_gather_into_tensor(gathered, packed, group=group)
+        else:
+            dist.all_gather(list(gathered.unbind(0)), packed, group=group)
     if gathered.is_cuda:
-        from . import _cabi
-        out = torch.empty(k, dtype=torch.float64, device=gathered.device)
-        with torch.cuda.device(gathered.device):
-            _cabi.check(_cabi.load().pnr_stats_merge_device(gathered.data_ptr(), world, k, out.data_ptr(),
-                                                            torch.cuda.current_stream(gathered.device).cuda_stream),
-                        "pnr_stats_merge_device")
+        _cabi.check(_cabi.load().pnr_stats_merge_device(gathered.data_ptr(), world, k, out.data_ptr(), stream),
+                    "pnr_stats_merge_device")
         return out
-    out = gathered.sum(0)
+    torch.sum(gathered, 0, out=out)
     out[4] = gathered[:, 4].max()
     out[5] = gathered[:, 5].min()
     return out
@@ -78,14 +83,14 @@ def reduce_packed(stats_local: torch.Tensor, extra_local: Optional[torch.Tensor]
     k = len(STATS_FIELDS)
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return stats_local.clone(), (None if extra_local is None else extra_local.clone())
-    world = dist.get_world_size(group)
-    packed = stats_local if extra_local is None else torch.cat([stats_local, extra_local])
-    gathered = torch.empty((world, packed.numel()), dtype=torch.float64, device=packed.device)
+    packed = (stats_local if extra_local is None else torch.cat([stats_local, extra_local])).contiguous()
+    gathered = packed.new_empty((dist.get_world_size(group), packed.numel()))
+    merged = torch.empty_like(packed)
     if packed.is_cuda:
-        dist.all_gather_into_tensor(gathered, packed.contiguous(), group=group)          # one NCCL all-gather
+        with torch.cuda.device(packed.device):
+            _gather_merge(packed, gathered, merged, group, torch.cuda.current_stream().cuda_stream)
     else:
-        dist.all_gather(list(gathered.unbind(0)), packed, group=group)                   # gloo
-    merged = _merge(gathered)
+        _gather_merge(packed, gathered, merged, group)
     return merged[:k], (None if extra_local is None else merged[k:].contiguous())
 
 
@@ -105,12 +110,13 @@ class IterationSync:
               The windows are plain cudaMalloc memory opened across processes with CUDA IPC; torch.distributed only carries
               the 64-byte handles, once, at construction.  No NCCL call in the step, so with ``cuda_graph=True`` the launch
               is captured and replayed at any world size.
-    ``nccl``  snapshot (pnr_stats_device [+ pnr_filter_delta_device]) -> all_gather_into_tensor -> pnr_stats_merge_device
-              [+ pnr_filter_sync_device]: five host calls.  Graph capture of this sequence would include the collective; it
-              is only attempted at world > 1 when ``PNR_GRAPH_COLLECTIVE=1``.
+    ``nccl``  snapshot (pnr_stats_device [+ pnr_filter_delta_device]) -> all_gather_into_tensor (world > 1) ->
+              pnr_stats_merge_device [+ pnr_filter_sync_device], the same gather-and-merge as ``reduce_packed``.  At
+              world > 1 it always runs eagerly: a communicator whose kernels live graphs still reference does not shut down
+              (DESIGN.md section 5).  At world 1 there is no collective and ``cuda_graph=True`` captures it.
 
     ``transport="auto"`` (default) uses p2p when every rank could open every other rank's window (same node, peer access)
-    and nccl otherwise; ``PNR_SYNC_TRANSPORT`` overrides.  ``__call__`` returns the merged float64[8] statistics tensor
+    and nccl otherwise.  A capture that fails raises.  ``__call__`` returns the merged float64[8] statistics tensor
     (device, not synchronised; valid until the next call).  A p2p wait that exceeds ``timeout_s`` yields NaN statistics and
     ``timed_out()`` reports it (a kernel never spins for ever on a dead peer); the ranks' sequence numbers may then disagree,
     so the next object must be built with ``reconnect=True`` on every rank (it re-opens the windows and restarts the
@@ -118,8 +124,6 @@ class IterationSync:
 
     def __init__(self, env, obs_filter=None, group: Optional[dist.ProcessGroup] = None, clear: bool = True,
                  cuda_graph: bool = False, transport: str = "auto", timeout_s: float = 20.0, reconnect: bool = False):
-        import os
-        from . import _cabi
         self.env, self.filter, self.group, self.clear = env, obs_filter, group, bool(clear)
         self._cabi, self._lib = _cabi, env._lib
         k = len(STATS_FIELDS)
@@ -132,10 +136,10 @@ class IterationSync:
         self._reconnect = bool(reconnect)
         dev = env.device
         self.packed = torch.zeros(self.len, dtype=torch.float64, device=dev)
-        self.gathered = torch.zeros((self.world, self.len), dtype=torch.float64, device=dev)
+        self.gathered = (torch.zeros((self.world, self.len), dtype=torch.float64, device=dev) if self.world > 1
+                         else self.packed.view(1, -1))
         self.merged = torch.zeros(self.len, dtype=torch.float64, device=dev)
         self._graph = None
-        transport = os.environ.get("PNR_SYNC_TRANSPORT", transport)
         if transport not in ("auto", "p2p", "nccl"):
             raise ValueError(f"unknown transport {transport!r}")
         self.transport = "p2p" if self.world == 1 and transport != "nccl" else transport
@@ -144,26 +148,11 @@ class IterationSync:
             if transport == "p2p" and self.transport != "p2p":
                 raise RuntimeError("IterationSync(transport='p2p'): the ranks could not open each other's windows: "
                                    + self._connect_error)
-        capture = cuda_graph and (self.transport == "p2p" or self.world == 1
-                                  or os.environ.get("PNR_GRAPH_COLLECTIVE") == "1")
-        if capture:
+        if cuda_graph and (self.transport == "p2p" or self.world == 1):
             with torch.cuda.device(dev):
-                # the communicator must exist before the capture; warm it with the (still empty) static buffers -- NOT with
-                # _run(), which clears the statistics window and merges the filter delta
-                if self.world > 1 and self.transport == "nccl":
-                    for _ in range(2):
-                        dist.all_gather_into_tensor(self.gathered, self.packed, group=self.group)
-                torch.cuda.synchronize(dev)
-                try:
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        self._run()
-                    self._graph = g
-                except Exception:  # noqa: BLE001 - capture of the collective is not available: stay eager
-                    if self.transport == "p2p":
-                        raise
-                    self._graph = None
-                    torch.cuda.synchronize(dev)
+                self._graph = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(self._graph):
+                    self._run()
 
     def _connect_windows(self) -> bool:
         """Exchange the CUDA IPC handles of the windows (one all-gather of 64 bytes per rank) and open the peers' windows;
@@ -207,13 +196,7 @@ class IterationSync:
         c.check(lib.pnr_stats_device(env._h, self.packed.data_ptr(), 1 if self.clear else 0, s), "pnr_stats_device")
         if self.filter is not None:
             c.check(lib.pnr_filter_delta_device(env._h, self.packed.data_ptr() + 8 * self.k, s), "pnr_filter_delta_device")
-        if self.world > 1:
-            dist.all_gather_into_tensor(self.gathered, self.packed, group=self.group)
-            src = self.gathered
-        else:
-            src = self.packed
-        c.check(lib.pnr_stats_merge_device(src.data_ptr(), self.world, self.len, self.merged.data_ptr(), s),
-                "pnr_stats_merge_device")
+        _gather_merge(self.packed, self.gathered, self.merged, self.group, s)
         if self.filter is not None:
             c.check(lib.pnr_filter_sync_device(env._h, self.merged.data_ptr() + 8 * self.k, s), "pnr_filter_sync_device")
 

@@ -167,27 +167,54 @@ def test_generic_chain_kernel_against_the_oracle(tmp_path):
 
 
 @pytest.mark.parametrize("chain", [0, 1])
-def test_less_specialised_kernels_agree_with_the_shipped_one(monkeypatch, chain):
-    """The shipped URDF runs pnr_step_dynamic_kernel<..., PIONEER_ISO>.  PNR_DYN_CHAIN forces the PIONEER (axis structure
-    only) and GENERIC (run-time axis codes) instantiations on the same robot: one env step from identical states must
-    land within the float32-vs-float64 bar of each other (all three are checked against the oracle on the CPU in
-    tests/test_dynamics_host.py)."""
+def test_less_specialised_kernels_agree_with_the_shipped_one(tmp_path, chain):
+    """The shipped URDF runs pnr_step_dynamic_kernel<..., PIONEER_ISO>; a modified copy of it selects a less specialised
+    instantiation from the robot model alone.
+    0, GENERIC (run-time axis codes): every joint limit widened to +-100 rad, beyond the +-64 rad of the PIONEER axis
+    pattern, with the same physics.  From states and PD set points well inside the shipped limits no joint stop engages,
+    so one env step from identical states lands within the float32-vs-float64 bar of the shipped kernel's.
+    1, PIONEER (axis structure only): arm1's centre of mass moved off its frame origin, so the composite bodies are no
+    longer isotropic.  The physics now differs from the shipped robot's: one env step is checked against the float64
+    oracle with the bars of test_one_step_against_the_float64_oracle.
+    (All three are checked against the oracle on the CPU in tests/test_dynamics_host.py.)"""
+    import re
+    from pioneer_b200.urdf import DEFAULT_URDF
+    text = open(DEFAULT_URDF).read()
+    if chain == 0:
+        text, count = re.subn(r'lower="[^"]+" upper="[^"]+"', 'lower="-100" upper="100"', text)
+    else:
+        text, count = re.subn(r'(<link name="robot:arm1"><inertial>)', r'\1<origin xyz="0.5 0 4"/>', text)
+    assert count == (6 if chain == 0 else 1)
+    path = tmp_path / "less_specialised.urdf"
+    path.write_text(text)
     n = 2048
     kw = dict(gravity=9.81, kp=800.0, kd=200.0, torque_scale=1e4)
     rng = np.random.default_rng(21)
     ref_env = make(n, seed=5, **kw)
-    q0 = rng.uniform(ref_env.r_lo * 0.9, ref_env.r_hi * 0.9, size=(n, 6)).astype(np.float32)
+    env = make(n, seed=5, urdf_path=str(path), **kw)
+    q0 = rng.uniform(ref_env.r_lo * 0.5, ref_env.r_hi * 0.5, size=(n, 6)).astype(np.float32)
     qd0 = (rng.normal(size=(n, 6)) * 0.5).astype(np.float32)
-    act = torch.as_tensor(rng.uniform(ref_env.r_lo, ref_env.r_hi, size=(n, 6)).astype(np.float32)).cuda()
-    ref_env.set_state(r=q0, v=qd0)
-    ref_env.step_tensor(act)
-    ref = ref_env.state()
-    monkeypatch.setenv("PNR_DYN_CHAIN", str(chain))
-    env = make(n, seed=5, **kw)
-    env.set_state(r=q0, v=qd0)
-    env.step_tensor(act)
-    got = env.state()
-    monkeypatch.delenv("PNR_DYN_CHAIN")
-    assert (got["r"] - ref["r"]).abs().max().item() <= 2e-5
-    assert (got["v"] - ref["v"]).abs().max().item() <= 2e-4
+    act = rng.uniform(ref_env.r_lo * 0.5, ref_env.r_hi * 0.5, size=(n, 6)).astype(np.float32)
+    for e in (ref_env, env):
+        e.set_state(r=q0, v=qd0)
+        obs = e.step_tensor(torch.as_tensor(act).cuda())[0]
+    ref, got = ref_env.state(), env.state()
+    if chain == 0:
+        assert (env.r_lo == -100).all() and (env.r_hi == 100).all()
+        lo, hi = torch.as_tensor(ref_env.r_lo).cuda(), torch.as_tensor(ref_env.r_hi).cuda()
+        assert ((ref["r"] > lo) & (ref["r"] < hi)).all()           # no joint stop engaged in either run
+        assert (got["r"] - ref["r"]).abs().max().item() <= 2e-5
+        assert (got["v"] - ref["v"]).abs().max().item() <= 2e-4
+    else:
+        assert np.abs(env.chain.body_com[1]).max() > 0
+        dyn, kin = chain_of(env)
+        cfg = DynConfig(**kw)
+        q1, qd1 = got["r"].cpu().numpy(), got["v"].cpu().numpy()
+        worst_q = worst_qd = worst_p = 0.0
+        for k in range(0, n, 16):
+            qo, qdo = dynamic_substeps(dyn, cfg, q0[k], qd0[k], act[k], env.r_lo, env.r_hi)
+            worst_q = max(worst_q, np.abs(q1[k] - qo).max())
+            worst_qd = max(worst_qd, np.abs(qd1[k] - qdo).max())
+            worst_p = max(worst_p, np.abs(obs[k, 126:129].cpu().numpy() - fk_pointer(kin, qo)).max())
+        assert worst_q <= 2e-5 and worst_qd <= 2e-4 and worst_p <= 5e-4, (worst_q, worst_qd, worst_p)
     ref_env.close(); env.close()
