@@ -5,7 +5,9 @@ requirements.txt:15 and not installable here, so this is written from the publis
 recurrence, ``var = S / (n - 1)`` for n > 1 else ``mean ** 2``, ``(x - mean) / (std + 1e-8)``, clip -- PARITY UNPINNED
 vs RLlib).  ``SequentialFilter`` is the reference-style filter (one observation at a time, statistics updated before the
 observation is normalised); ``BatchSyncFilter`` is the semantics of pnr_filter_apply / pnr_filter_sync (statistics
-pushed per batch, normalisation with the statistics of the last synchronisation)."""
+pushed per batch, normalisation with the statistics of the last synchronisation).  Both take RLlib's ``demean`` / ``destd``
+flags: the mean is subtracted only if ``demean``, the result divided by ``std + 1e-8`` only if ``destd``; the running
+statistics are kept either way."""
 from __future__ import annotations
 
 import numpy as np
@@ -35,20 +37,22 @@ class RunningStat:
 
 
 class SequentialFilter:
-    def __init__(self, dim, clip=10.0):
-        self.rs, self.clip = RunningStat(dim), clip
+    def __init__(self, dim, clip=10.0, demean=True, destd=True):
+        self.rs, self.clip, self.demean, self.destd = RunningStat(dim), clip, demean, destd
 
     def __call__(self, x, update=True):
         x = np.asarray(x, np.float64)
         if update:
             self.rs.push(x)
-        y = (x - self.rs.M) / (self.rs.std + 1e-8)
+        y = x - self.rs.M if self.demean else x
+        if self.destd:
+            y = y / (self.rs.std + 1e-8)
         return np.clip(y, -self.clip, self.clip)
 
 
 class BatchSyncFilter:
-    def __init__(self, dim, clip=10.0):
-        self.rs, self.clip = RunningStat(dim), clip
+    def __init__(self, dim, clip=10.0, demean=True, destd=True):
+        self.rs, self.clip, self.demean, self.destd = RunningStat(dim), clip, demean, destd
         # before the first synchronisation nothing has been pushed: the filter is the identity (mean 0, scale 1), as an
         # RLlib filter that has seen no sample never normalises anything
         self.applied_mean, self.applied_std = np.zeros(dim), np.ones(dim) - 1e-8
@@ -58,9 +62,11 @@ class BatchSyncFilter:
         batch = np.asarray(batch, np.float64)
         if update:
             self.pending.append(batch.copy())
-        mean32 = self.applied_mean.astype(np.float32).astype(np.float64)      # the device applies float32 statistics
-        inv32 = (1.0 / (self.applied_std + 1e-8)).astype(np.float32).astype(np.float64)
-        y = (batch - mean32) * inv32
+        y = batch                                   # the device applies float32 statistics
+        if self.demean:
+            y = y - self.applied_mean.astype(np.float32).astype(np.float64)
+        if self.destd:
+            y = y * (1.0 / (self.applied_std + 1e-8)).astype(np.float32).astype(np.float64)
         return np.clip(y, -self.clip, self.clip)
 
     def sync(self):
